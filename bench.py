@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the receive-chain hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1], "c2"): IQBaseBand<float>(64 taps, shift 100 kHz, 20 MS/s ->
@@ -19,6 +19,12 @@ steady state.  Metric: input IQ Msamples/s.
   c5_bank  : BASELINE configs[4], the 2048-channel int16 bank sharded over the ranks (strong
              scaling), every rank's FM/AM rows stored straight into rank 0's HBM, with a bit-exact
              check of the gathered spot channels against the oracle outside the timed region
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed pass returned -- the
+base band (n, 2) and the demodulated audio (n,), float32 -- as DIR/baseband.npy and DIR/audio.npy
+(above DUMP_LIMIT bytes in all, the same seeded sample of rows of both, plus DIR/sample_index.npy).
+The input is seeded and the chain state depends only on the arguments, so two builds run with the
+same arguments can be compared output for output.
 
 N > 1: one process per GPU.  C2: every rank runs its own independent stream (weak scaling, no
 data-path collective).  The demodulated audio of all ranks is gathered on rank 0 WITHOUT a
@@ -49,6 +55,7 @@ METRIC = "iq_msamples_per_s_iqbaseband_fmdemod"
 UNIT = "Msamples/s"
 G_BATCH = 8                       # passes per progress flag / per NCCL collective
 C5_SPOT = (0, 1, 1023, 1024, 1025, 2047, 389, 1707)
+DUMP_LIMIT = 64 * 10 ** 6         # bytes written by --dump-outputs at most
 
 
 def workload():
@@ -522,6 +529,20 @@ def secondary_workloads(coll, dev, x_c2):
     return out
 
 
+def dump_outputs(path, arrays):
+    """Writes path/<name>.npy for each (n, ...) array of `arrays`; above DUMP_LIMIT bytes in all, the same
+    seeded sample of rows of every array, and its row numbers as sample_index.npy."""
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    if n * row_bytes > DUMP_LIMIT:
+        m = (DUMP_LIMIT - 4096) // (row_bytes + 8)                      # 4096: room for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+        arrays = dict({k: a[idx] for k, a in arrays.items()}, sample_index=idx.astype(np.float64))
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def hbm_peak():
     peaks = {}
     try:
@@ -562,7 +583,10 @@ def main():
     ap.add_argument("--buffers", type=int, default=0, help="buffers per pass (default: the workload's n_buffers)")
     ap.add_argument("--passes", type=int, default=int(os.environ.get("SDRG_BENCH_PASSES", "80")),
                     help="passes over the 2 GiB batch per step (rounded up to a multiple of %d)" % G_BATCH)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed pass as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         reference_arm(args)
         return
@@ -591,7 +615,7 @@ def main():
     dev = torch.device("cuda", local)
     coll = Collective(dist, world, dev)
     W = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
     R = max(G_BATCH, (max(args.passes, 1) + G_BATCH - 1) // G_BATCH * G_BATCH)
 
     c = workload()
@@ -637,6 +661,7 @@ def main():
     pending = [None, None]
     cons = torch.cuda.Stream(device=dev) if (win is not None and rank == 0) else None
     counter = [0]
+    last = [None]                                            # what the latest pass returned (--dump-outputs)
 
     # Per-kernel CUDA events (sdrg_profile) are recorded on every 16th pass of the timed region: the event
     # records between the kernels cost ~3 % of a pass when taken on every one.
@@ -657,7 +682,7 @@ def main():
             if slot == 0 and b >= 2:
                 win.wait(win.ack(), 1, b - 1, stream_ptr())             # the consumer released this ring
             audio = win.base + win.data_offset + (((rank * 2 + ring) * G + slot) * cap) * 4
-            chain.process_into(x_dev, bs, bb_out.data_ptr(), audio, cap)
+            last[0] = (chain.process_into(x_dev, bs, bb_out.data_ptr(), audio, cap), audio - win.base)
             if slot == G - 1:
                 win.signal(win.slot(rank), b + 1, stream_ptr())
                 if cons is not None:                                     # rank 0's consumer stream: all rows of batch b are in
@@ -668,7 +693,7 @@ def main():
         if slot == 0 and pending[ring] is not None:
             pending[ring].wait()                    # the gather that last read this ring has finished
             pending[ring] = None
-        chain.process(x_dev, bs, bb_out=bb_out, audio_out=rings[ring][slot])
+        last[0] = chain.process(x_dev, bs, bb_out=bb_out, audio_out=rings[ring][slot])
         if world > 1 and slot == G - 1:
             pending[ring] = dist.all_gather_into_tensor(gathered2[ring], rings[ring], async_op=True)
 
@@ -726,6 +751,13 @@ def main():
     ms = coll.max(ev0.elapsed_time(ev1))
     acc_ms, acc_n = _lib.profile_read(_lib.KERNEL_IQBB_ACCUM)
     fin_ms, fin_n = _lib.profile_read(_lib.KERNEL_IQBB_FINALIZE)
+    if args.dump_outputs and rank == 0:
+        if win is not None:                                  # rank 0's audio lies in its own peer window
+            got, off = last[0]
+            yb, ya = bb_out[:got].cpu().numpy(), win.read(off, got * 4).view(np.float32)
+        else:
+            yb, ya = (t.cpu().numpy() for t in last[0][:2])
+        dump_outputs(args.dump_outputs, {"baseband": yb, "audio": ya})
     if win is not None and win.timed_out():
         raise SystemExit("bench.py: a peer-window wait timed out")
     value = world * n_pass * R * K / (ms * 1e-3) / 1e6

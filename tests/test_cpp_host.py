@@ -115,22 +115,30 @@ def test_wav_to_wav_real_baseband_fm_chain(tmp_path):
 
 @pytest.mark.parametrize("typ,dt,ncomp", [("u8", "uint8", 1), ("s16", "int16", 1), ("cu8", "uint8", 2), ("cs16", "int16", 2)])
 def test_wav_nodes_vs_live_reference(typ, dt, ncomp, tmp_path):
-    """Random payload, odd sizes: file written by the reference's WavSink (prebuilt harness) == file written by ours,
-    and both sources deliver the same buffers."""
+    """Random payload, odd sizes: the file our WavSink writes and the buffers our WavSource delivers == the reference's
+    (its recorded outputs, tests/recorded.py; and its WavSink/WavSource themselves when oracle/_ref/ref_harness is built)."""
     import numpy as np
+    import recorded
     harness = os.path.join(ROOT, "oracle", "_ref", "ref_harness")
-    if not os.path.exists(harness):
-        pytest.skip("oracle/_ref/ref_harness not built")
     g = np.random.default_rng(len(typ) * 7 + ncomp)
     frames, bs, Fs = int(g.integers(1500, 5000)), int(g.choice([333, 1024, 4000])), float(g.choice([8000.0, 44100.0, 2.4e6]))
     info = np.iinfo(dt)
     x = g.integers(info.min, info.max + 1, size=frames * ncomp).astype(dt)
     inp, ref, pre, mine = tmp_path / "in.raw", tmp_path / "ref.wav", tmp_path / "ref", tmp_path / "mine"
     x.tofile(inp)
-    subprocess.run([harness, "wav", typ, str(inp), str(bs), repr(Fs), str(ref), str(pre)], check=True)
+    live = os.path.exists(harness)
+    if live:
+        subprocess.run([harness, "wav", typ, str(inp), str(bs), repr(Fs), str(ref), str(pre)], check=True)
+    # without the reference's build, our WavSource reads the file our WavSink has just written, whose bytes the
+    # recorded digest pins to the reference's file
     exe = compile_cpp("wav_test")
-    r = subprocess.run([exe, typ, str(inp), str(bs), repr(Fs), str(ref), str(mine)], capture_output=True, text=True, timeout=60)
+    src = str(ref) if live else str(mine) + ".wav"
+    r = subprocess.run([exe, typ, str(inp), str(bs), repr(Fs), src, str(mine)], capture_output=True, text=True, timeout=60)
     assert r.returncode == 0, r.stdout + r.stderr
-    np.testing.assert_array_equal(np.fromfile(str(mine) + ".wav", dtype=np.uint8), np.fromfile(str(ref), dtype=np.uint8))
-    for ext, t in ((".data", np.uint8), (".counts", np.uint32), (".cfg", np.float64)):
-        np.testing.assert_array_equal(np.fromfile(str(mine) + ext, dtype=t), np.fromfile(str(pre) + ext, dtype=t))
+    outs = {ext[1:]: np.fromfile(str(mine) + ext, dtype=t)
+            for ext, t in ((".wav", np.uint8), (".data", np.uint8), (".counts", np.uint32), (".cfg", np.float64))}
+    recorded.check("wav_" + typ, **outs)
+    if live:
+        np.testing.assert_array_equal(outs["wav"], np.fromfile(str(ref), dtype=np.uint8))
+        for ext, t in ((".data", np.uint8), (".counts", np.uint32), (".cfg", np.float64)):
+            np.testing.assert_array_equal(outs[ext[1:]], np.fromfile(str(pre) + ext, dtype=t))

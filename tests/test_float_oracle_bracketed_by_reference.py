@@ -2,9 +2,11 @@
 
 IQBaseBand<float> does not compile and FMDemod<float> does not link in the reference, so the float path's
 semantics are defined by oracle/sdr_oracle.c ("parity unpinned").  This test turns "defined" into "bounded by
-the reference": the same int16-valued samples go through the REFERENCE's IQBaseBand<int16_t> (+ FMDemod, the
-prebuilt oracle/_ref/ref_harness; nothing under /root/reference is read) and through the float oracle, and the
-two must agree to within the integer path's own truncation errors, stage by stage:
+the reference": the same int16-valued samples go through the reference's IQBaseBand<int16_t> (+ FMDemod) and
+through the float oracle, and the two must agree to within the integer path's own truncation errors, stage by
+stage.  The integer side is the int16 oracle, pinned bit-exact to the reference by test_oracle_vs_golden.py and
+test_oracle_vs_live_reference.py; its outputs here are checked against recorded digests (tests/recorded.py) and,
+when oracle/_ref/ref_harness (the reference's build) is present, against the reference itself:
 
   taps     k_i = trunc(2^14 a_i)        float uses a_i           |dk| < 2^-14 per component  (baseband.hh:260)
   FIR      y = (sum k x) >> 14          floor per component      <= 1
@@ -26,12 +28,12 @@ import subprocess
 import numpy as np
 import pytest
 
+import recorded
 from conftest import ROOT
 from libsdr_b200 import synth
 from oracle import oracle as orc
 
 HARNESS = os.path.join(ROOT, "oracle", "_ref", "ref_harness")
-pytestmark = pytest.mark.skipif(not os.path.exists(HARNESS), reason="oracle/_ref/ref_harness not built")
 
 #        name            Fs      Fc       Ff       width   order  ss  oFs      amplitude
 CASES = [("c1",          2.4e6,  100e3,   100e3,   12.5e3, 15,    1,  48000.0, 8192),
@@ -55,18 +57,30 @@ def test_float_oracle_within_truncation_bound_of_reference_int16(case, tmp_path)
     n, bs = 60000, 20000
     x = _signal(n, Fs, Fc, amp, 77 + order)
     A = float(np.abs(x.astype(np.int64)).max())
-    inp = tmp_path / "x.bin"; x.tofile(inp)
-    pre = str(tmp_path / "out")
-    subprocess.run([HARNESS, "bb", "s16", str(inp), str(bs), repr(Fs), repr(Fc), repr(Ff), repr(width), str(order), str(ss),
-                    repr(oFs), "0", pre], check=True)
-    ref_bb = np.fromfile(pre + ".bb", dtype=np.int16).reshape(-1, 2).astype(np.float64)
-    ref_fm = np.fromfile(pre + ".fm", dtype=np.int16).astype(np.float64)
-    counts = np.fromfile(pre + ".counts", dtype=np.uint32)
+
+    # the integer chain, buffer by buffer
+    oi = orc.IQBaseBand(orc.S16, Fc, Ff, width, order, ss, oFs); oi.config(Fs, bs)
+    oifm = orc.FMDemod(orc.S16)
+    i_bb, i_fm, counts = [], [], []
+    for k in range(0, n, bs):
+        y = oi.process(x[k:k + bs]); counts.append(y.shape[0])
+        if y.shape[0]:
+            i_bb.append(y); i_fm.append(oifm.process(y, inplace=True))
+    counts, i_bb, i_fm = np.array(counts, dtype=np.uint32), np.concatenate(i_bb), np.concatenate(i_fm)
+    recorded.check("bracket_" + name, counts=counts, bb=i_bb, fm=i_fm)
+    if os.path.exists(HARNESS):
+        inp = tmp_path / "x.bin"; x.tofile(inp)
+        pre = str(tmp_path / "out")
+        subprocess.run([HARNESS, "bb", "s16", str(inp), str(bs), repr(Fs), repr(Fc), repr(Ff), repr(width), str(order), str(ss),
+                        repr(oFs), "0", pre], check=True)
+        np.testing.assert_array_equal(counts, np.fromfile(pre + ".counts", dtype=np.uint32))
+        np.testing.assert_array_equal(i_bb, np.fromfile(pre + ".bb", dtype=np.int16).reshape(-1, 2))
+        np.testing.assert_array_equal(i_fm, np.fromfile(pre + ".fm", dtype=np.int16))
+    ref_bb, ref_fm = i_bb.astype(np.float64), i_fm.astype(np.float64)
 
     # the float oracle on the same sample VALUES
     of = orc.IQBaseBand(orc.F32, Fc, Ff, width, order, ss, oFs); of.config(Fs, bs)
     ofm = orc.FMDemod(orc.F32)
-    oi = orc.IQBaseBand(orc.S16, Fc, Ff, width, order, ss, oFs); oi.config(Fs, bs)      # for the integer tables only
     f_bb, f_fm, first, f_counts = [], [], [], []
     off = 0
     for k in range(0, n, bs):
