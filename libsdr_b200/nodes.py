@@ -439,21 +439,23 @@ class FilterNode:
         return n.value
 
     def process(self, x):
-        F = max(self.n_filters(), 1)
+        """Without filters the stream still advances (history, pending samples), and the result has no rows, like a
+        FilterSink without sources."""
+        F = self.n_filters()
         got = C.c_size_t(0)
         if _is_torch(x):
             import torch
             n_in = x.shape[0]
             n_out = self.outputs_for(n_in)
-            out = torch.empty((F, max(n_out, 1)), dtype=torch.complex64, device=x.device)
+            out = torch.empty((max(F, 1), max(n_out, 1)), dtype=torch.complex64, device=x.device)
             _lib.call("sdrg_filter_process_dev", self._h, _dev_in(x, np.complex64), n_in, C.c_void_p(out.data_ptr()),
                       max(n_out, 1), C.byref(got), _stream_ptr())
-            return out[:, :got.value]
+            return out[:F, :got.value]
         x = np.ascontiguousarray(x, dtype=np.complex64).reshape(-1)
         n_out = self.outputs_for(x.shape[0])
-        out = np.zeros((F, max(n_out, 1)), dtype=np.complex64)
+        out = np.zeros((max(F, 1), max(n_out, 1)), dtype=np.complex64)
         _lib.call("sdrg_filter_process", self._h, _np_ptr(x), x.shape[0], _np_ptr(out), max(n_out, 1), C.byref(got))
-        return out[:, :got.value]
+        return out[:F, :got.value]
 
 
 class ChannelBank:
