@@ -258,7 +258,10 @@ int sdrg_filter_process_dev(sdrg_filter *h, const void *d_in, size_t n_in, void 
 /* ---- channel bank: C independent IQBaseBand<Scalar> nodes on ONE input stream, each followed by
  *      FM / AM / USB demodulators connected out of place (several sinks on one source,
  *      src/node.cc:75).  Channel c equals IQBaseBand<Scalar>(Fc[c], Ff[c], width, order, sub_sample, oFs)
- *      (src/baseband.hh:47-57) bit for bit; Ff == NULL means Ff = Fc.  scalar: SDRG_T_S8 / SDRG_T_S16.
+ *      (src/baseband.hh:47-57) bit for bit; Ff == NULL means Ff = Fc.  scalar: SDRG_T_S8 / SDRG_T_S16, or
+ *      SDRG_T_F32: input complex float, outputs as sdrg_rxchain's float chain (base band float2, FM / AM /
+ *      USB float), each channel equal to the float node to float rounding; sdrg_bank_get_info then returns
+ *      float taps (as sdrg_iqbb_get_info).  Every scalar needs sub_sample >= 256 and order <= 256.
  *      Outputs of channel c land at <ptr> + c*out_stride elements; any output pointer may be NULL. -- */
 typedef struct sdrg_bank sdrg_bank;
 int sdrg_bank_create(int scalar, size_t n_channels, const double *Fc, const double *Ff, double width, size_t order,
@@ -280,7 +283,8 @@ int sdrg_bank_process_dev(sdrg_bank *h, const void *d_in, size_t buffer_size, si
  *
  * (1) One process, G devices: a channel bank whose channels are sharded by contiguous ranges over
  *     `devices` (shard g owns channels [g*C/G, (g+1)*C/G), the first C%G shards one more).  Same
- *     semantics and bit-identical results as sdrg_bank_* with all channels on one device.
+ *     semantics and bit-identical results as sdrg_bank_* with all channels on one device (int8, int16;
+ *     SDRG_T_F32 is accepted too, each shard being a float bank, equal to it to float rounding).
  *     _process:     host pointers; every device uploads the input and returns its rows; blocking.
  *     _process_dev: input and output arrays live on devices[0]; `stream` is a stream of devices[0]; the
  *                   input is broadcast with copy-engine peer copies, shards with peer access store their

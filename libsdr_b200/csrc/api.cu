@@ -205,28 +205,8 @@ int upload_fold_tables(sdrg_iqbb *h) {
   const bool nco = d.lut_inc != 0, neg = d.negative;
   const uint64_t inc = d.lut_inc & 0x7fffu;
   std::vector<float> A(2 * 128), U(2 * 256 * L);
-  for (size_t a = 0; a < 128; ++a) {
-    A[2 * a] = nco ? (float)d.lutd_re[a] : 1.0f;
-    A[2 * a + 1] = nco ? (float)(neg ? -d.lutd_im[a] : d.lutd_im[a]) : 0.0f;
-  }
-  std::vector<double> br(L), bi(L);
-  for (size_t r = 0; r < 256; ++r) {
-    for (size_t j = 0; j < L; ++j) {           // B(r, j)
-      if (!nco) { br[j] = 1.0; bi[j] = 0.0; continue; }
-      const uint64_t s = (r + j * inc) >> 8;
-      const size_t idx = neg ? (size_t)((127 + 128 - (s % 128)) % 128) : (size_t)(s % 128);
-      br[j] = d.lutd_re[idx]; bi[j] = d.lutd_im[idx];
-    }
-    for (size_t e = 0; e < L; ++e) {
-      double sr = 0, si = 0;
-      for (size_t j = 0; j + e < L; ++j) {
-        const double kr = d.kd_re[L - 1 - e - j], ki = d.kd_im[L - 1 - e - j];
-        sr += br[j] * kr - bi[j] * ki;
-        si += br[j] * ki + bi[j] * kr;
-      }
-      U[2 * (r * L + e)] = (float)sr; U[2 * (r * L + e) + 1] = (float)si;
-    }
-  }
+  fold_table_a(d, nco, neg, A.data());
+  fold_table_u(d, L, U.data());
   SDRG_CUDA(cudaMalloc(&h->d_tab_a, A.size() * sizeof(float)));
   SDRG_CUDA(cudaMemcpy(h->d_tab_a, A.data(), A.size() * sizeof(float), cudaMemcpyHostToDevice));
   SDRG_CUDA(cudaMalloc(&h->d_tab_u, U.size() * sizeof(float)));

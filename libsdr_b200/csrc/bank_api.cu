@@ -1,7 +1,8 @@
 // bank_api.cu -- C ABI of the channel bank: C independent IQBaseBand<Scalar> chains on one input
 // stream, each followed by FM / AM / USB demodulators connected out of place (several sinks on one
 // source, src/node.cc:75), i.e. BASELINE configs 4 and 5.  Per channel the results are bit-identical
-// to an IQBaseBand<Scalar>(Fc_k, Ff_k, width, order, sub_sample, oFs) node fed the same buffers.
+// to an IQBaseBand<Scalar>(Fc_k, Ff_k, width, order, sub_sample, oFs) node fed the same buffers (int8 / int16);
+// float channels match the float node to rounding (folded weights, bank_fold_f32_kernel).
 #include "iqbb_kernels.cuh"
 
 #include <vector>
@@ -14,7 +15,7 @@ struct sdrg_bank {
   std::vector<IqbbDesign> d;
   bool configured = false;
   uint32_t taps_len = 1, hist_len = 0;
-  void *d_taps = nullptr, *d_lut = nullptr, *d_inc = nullptr, *d_neg = nullptr;
+  void *d_taps = nullptr, *d_lut = nullptr, *d_inc = nullptr, *d_neg = nullptr, *d_tab_u = nullptr;
   void *d_hist[2] = {nullptr, nullptr};
   void *d_acc[2] = {nullptr, nullptr};
   size_t acc_stride = 0; uint32_t acc_dirty[2] = {0, 0};
@@ -29,6 +30,7 @@ struct sdrg_bank {
 
 namespace {
 size_t sample_bytes(int scalar) { return 2 * scalar_bytes(scalar); }
+size_t fm_bytes(int scalar) { return scalar == SDRG_T_F32 ? 4 : 2; }
 void free_dev(void **p) { if (*p) { cudaFree(*p); *p = nullptr; } }
 
 int ensure_acc(sdrg_bank *h, size_t slots) {
@@ -64,7 +66,7 @@ int sdrg_bank_create(int scalar, size_t n_channels, const double *Fc, const doub
                      size_t sub_sample, double oFs, sdrg_bank **out) {
   if (!out || !Fc) return set_error(SDRG_ERR_ARG, "null argument");
   *out = nullptr;
-  if (scalar != SDRG_T_S8 && scalar != SDRG_T_S16) return set_error(SDRG_ERR_ARG, "bank: scalar must be int8 or int16");
+  if (scalar != SDRG_T_S8 && scalar != SDRG_T_S16 && scalar != SDRG_T_F32) return set_error(SDRG_ERR_ARG, "bank: scalar must be int8, int16 or float");
   if (n_channels == 0) return set_error(SDRG_ERR_ARG, "bank: no channels");
   if (order > 256) return set_error(SDRG_ERR_ARG, "bank: order %zu exceeds 256", order);
   sdrg_bank *h = new sdrg_bank();
@@ -78,8 +80,8 @@ int sdrg_bank_create(int scalar, size_t n_channels, const double *Fc, const doub
     d.Fc = int32_t(Fc[c]); d.Ff = int32_t(Ff ? Ff[c] : Fc[c]); d.Fs = 0; d.width = int32_t(width);
     d.order = order < 1 ? 1 : order;
     d.sub_sample = sub_sample; d.oFs = oFs;
+    design_lut(d);
   }
-  design_lut(h->d[0]);
   *out = h;
   return SDRG_OK;
 }
@@ -88,7 +90,7 @@ int sdrg_bank_destroy(sdrg_bank *h) {
   if (!h) return SDRG_OK;
   cudaSetDevice(h->device); cudaDeviceSynchronize();
   if (h->stream) cudaStreamDestroy(h->stream);
-  free_dev(&h->d_taps); free_dev(&h->d_lut); free_dev(&h->d_inc); free_dev(&h->d_neg);
+  free_dev(&h->d_taps); free_dev(&h->d_lut); free_dev(&h->d_inc); free_dev(&h->d_neg); free_dev(&h->d_tab_u);
   free_dev(&h->d_hist[0]); free_dev(&h->d_hist[1]); free_dev(&h->d_acc[0]); free_dev(&h->d_acc[1]);
   free_dev(&h->d_fm_last[0]); free_dev(&h->d_fm_last[1]); free_dev(&h->d_in);
   for (int k = 0; k < 4; ++k) free_dev(&h->d_out[k]);
@@ -120,24 +122,43 @@ int sdrg_bank_configure(sdrg_bank *h, const sdrg_config *src, sdrg_config *out) 
     if (d.lut_inc > 0xffffffffull) return set_error(SDRG_ERR_CONFIG, "bank: NCO increment out of range");
     ss = d.sub_sample;
     size_t l = 0;
-    while (l + 1 < L && d.k_re[l] == 0 && d.k_im[l] == 0) ++l;
+    if (h->scalar != SDRG_T_F32) while (l + 1 < L && d.k_re[l] == 0 && d.k_im[l] == 0) ++l;
     if (l < lead) lead = l;
   }
   if (ss < 256) return set_error(SDRG_ERR_CONFIG, "bank: the bank kernel needs sub-sampling >= 256 (got %zu); use IQBaseBand nodes", ss);
   if (ss > (1u << 30)) return set_error(SDRG_ERR_CONFIG, "bank: sub-sampling %zu too large", ss);
-  const size_t Lp = L - lead;      // common leading zero taps are dropped (exact)
-  std::vector<int32_t> taps(4 * Lp * C), lut(256);
-  for (size_t c = 0; c < C; ++c)
-    for (size_t i = 0; i < Lp; ++i) {
-      const uint32_t kr = (uint32_t)h->d[c].k_re[lead + i], ki = (uint32_t)h->d[c].k_im[lead + i];
-      int32_t *t = &taps[4 * (c * Lp + i)];
-      t[0] = (int32_t)kr; t[1] = (int32_t)(ki - kr); t[2] = (int32_t)(kr + ki); t[3] = 0;
-    }
-  for (size_t j = 0; j < 128; ++j) { lut[2 * j] = h->d[0].lut_re[j]; lut[2 * j + 1] = h->d[0].lut_im[j]; }
-  free_dev(&h->d_taps); free_dev(&h->d_lut); free_dev(&h->d_inc); free_dev(&h->d_neg);
+  const size_t Lp = L - lead;      // common leading zero taps are dropped (exact; integer taps only)
+  free_dev(&h->d_taps); free_dev(&h->d_lut); free_dev(&h->d_inc); free_dev(&h->d_neg); free_dev(&h->d_tab_u);
   free_dev(&h->d_hist[0]); free_dev(&h->d_hist[1]);
-  SDRG_CUDA(cudaMalloc(&h->d_taps, taps.size() * 4)); SDRG_CUDA(cudaMemcpy(h->d_taps, taps.data(), taps.size() * 4, cudaMemcpyHostToDevice));
-  SDRG_CUDA(cudaMalloc(&h->d_lut, 1024)); SDRG_CUDA(cudaMemcpy(h->d_lut, lut.data(), 1024, cudaMemcpyHostToDevice));
+  if (h->scalar == SDRG_T_F32) {
+    // bank_fold_f32_kernel: taps [t][channel] and U_c(r, 0) [group][r][channel in group], channels padded to 32 with zeros
+    const size_t Cp = (C + 31) / 32 * 32;
+    std::vector<float> taps(2 * L * Cp, 0.0f), tab_u(2 * 256 * Cp, 0.0f), u(2 * 256), lut(256);
+    for (size_t c = 0; c < C; ++c) {
+      const IqbbDesign &d = h->d[c];
+      for (size_t t = 0; t < L; ++t) { taps[2 * (t * Cp + c)] = (float)d.kd_re[t]; taps[2 * (t * Cp + c) + 1] = (float)d.kd_im[t]; }
+      fold_table_u(d, 1, u.data());
+      for (size_t r = 0; r < 256; ++r) {
+        const size_t k = ((c / 32) * 256 + r) * 32 + c % 32;
+        tab_u[2 * k] = u[2 * r]; tab_u[2 * k + 1] = u[2 * r + 1];
+      }
+    }
+    for (size_t j = 0; j < 128; ++j) { lut[2 * j] = (float)h->d[0].lutd_re[j]; lut[2 * j + 1] = (float)h->d[0].lutd_im[j]; }
+    SDRG_CUDA(cudaMalloc(&h->d_taps, taps.size() * 4)); SDRG_CUDA(cudaMemcpy(h->d_taps, taps.data(), taps.size() * 4, cudaMemcpyHostToDevice));
+    SDRG_CUDA(cudaMalloc(&h->d_tab_u, tab_u.size() * 4)); SDRG_CUDA(cudaMemcpy(h->d_tab_u, tab_u.data(), tab_u.size() * 4, cudaMemcpyHostToDevice));
+    SDRG_CUDA(cudaMalloc(&h->d_lut, 1024)); SDRG_CUDA(cudaMemcpy(h->d_lut, lut.data(), 1024, cudaMemcpyHostToDevice));
+  } else {
+    std::vector<int32_t> taps(4 * Lp * C), lut(256);
+    for (size_t c = 0; c < C; ++c)
+      for (size_t i = 0; i < Lp; ++i) {
+        const uint32_t kr = (uint32_t)h->d[c].k_re[lead + i], ki = (uint32_t)h->d[c].k_im[lead + i];
+        int32_t *t = &taps[4 * (c * Lp + i)];
+        t[0] = (int32_t)kr; t[1] = (int32_t)(ki - kr); t[2] = (int32_t)(kr + ki); t[3] = 0;
+      }
+    for (size_t j = 0; j < 128; ++j) { lut[2 * j] = h->d[0].lut_re[j]; lut[2 * j + 1] = h->d[0].lut_im[j]; }
+    SDRG_CUDA(cudaMalloc(&h->d_taps, taps.size() * 4)); SDRG_CUDA(cudaMemcpy(h->d_taps, taps.data(), taps.size() * 4, cudaMemcpyHostToDevice));
+    SDRG_CUDA(cudaMalloc(&h->d_lut, 1024)); SDRG_CUDA(cudaMemcpy(h->d_lut, lut.data(), 1024, cudaMemcpyHostToDevice));
+  }
   SDRG_CUDA(cudaMalloc(&h->d_inc, C * 4)); SDRG_CUDA(cudaMemcpy(h->d_inc, inc.data(), C * 4, cudaMemcpyHostToDevice));
   SDRG_CUDA(cudaMalloc(&h->d_neg, C * 4)); SDRG_CUDA(cudaMemcpy(h->d_neg, neg.data(), C * 4, cudaMemcpyHostToDevice));
   h->taps_len = (uint32_t)Lp; h->hist_len = (uint32_t)Lp - 1;
@@ -171,7 +192,12 @@ int sdrg_bank_get_info(const sdrg_bank *h, size_t *channels, size_t *sub_sample,
     info->order = d.order; info->sub_sample = d.sub_sample; info->lut_inc = d.lut_inc; info->negative_shift = d.negative ? 1 : 0;
     info->samples_consumed = h->consumed; info->outputs_produced = windows_done(h->consumed, d.sub_sample);
   }
-  if (kernel) for (size_t i = 0; i < d.order; ++i) { ((int32_t *)kernel)[2 * i] = d.k_re[i]; ((int32_t *)kernel)[2 * i + 1] = d.k_im[i]; }
+  if (kernel) {
+    for (size_t i = 0; i < d.order; ++i) {
+      if (h->scalar == SDRG_T_F32) { ((float *)kernel)[2 * i] = (float)d.kd_re[i]; ((float *)kernel)[2 * i + 1] = (float)d.kd_im[i]; }
+      else { ((int32_t *)kernel)[2 * i] = d.k_re[i]; ((int32_t *)kernel)[2 * i + 1] = d.k_im[i]; }
+    }
+  }
   return SDRG_OK;
 }
 
@@ -203,7 +229,7 @@ int sdrg_bank_process_dev(sdrg_bank *h, const void *d_in, size_t buffer_size, si
   const int p = h->parity, q = p ^ 1;
   BankAccumArgs a{};
   a.x = d_in; a.hist_in = h->d_hist[p]; a.hist_out = h->d_hist[q];
-  a.taps = h->d_taps; a.lut = h->d_lut; a.inc = (const uint32_t *)h->d_inc; a.neg = (const uint32_t *)h->d_neg;
+  a.taps = h->d_taps; a.lut = h->d_lut; a.tab_u = h->d_tab_u; a.inc = (const uint32_t *)h->d_inc; a.neg = (const uint32_t *)h->d_neg;
   a.acc_cur = h->d_acc[p]; a.acc_next = h->d_acc[q]; a.acc_stride = h->acc_stride;
   a.n = (uint32_t)n_in; a.channels = (uint32_t)h->channels; a.group = 32;
   a.taps_len = h->taps_len; a.hist_len = h->hist_len; a.ss = (uint32_t)ss; a.r0 = adv.r0; a.first = adv.first;
@@ -216,7 +242,7 @@ int sdrg_bank_process_dev(sdrg_bank *h, const void *d_in, size_t buffer_size, si
   f.fm_last_in = h->d_fm_last[h->fm_parity]; f.fm_last_out = h->d_fm_last[h->fm_parity ^ 1];
   BankFinalizeStrides s{h->acc_stride, out_stride, (uint32_t)sample_bytes(h->scalar), 0};
   bool bb_done = false, any = false;
-  struct { void *ptr; int demod; uint32_t bytes; } outs[3] = {{d_fm, SDRG_DEMOD_FM, 2}, {d_am, SDRG_DEMOD_AM, (uint32_t)scalar_bytes(h->scalar)},
+  struct { void *ptr; int demod; uint32_t bytes; } outs[3] = {{d_fm, SDRG_DEMOD_FM, (uint32_t)fm_bytes(h->scalar)}, {d_am, SDRG_DEMOD_AM, (uint32_t)scalar_bytes(h->scalar)},
                                                              {d_usb, SDRG_DEMOD_USB, (uint32_t)scalar_bytes(h->scalar)}};
   for (int k = 0; k < 3; ++k) {
     if (!outs[k].ptr) continue;
@@ -248,7 +274,7 @@ int sdrg_bank_process(sdrg_bank *h, const void *in, size_t buffer_size, size_t n
   int rc = grow(&h->d_in, &h->in_cap, n_in * sb);
   if (rc) return rc;
   void *host[4] = {bb, fm, am, usb};
-  const size_t eb[4] = {sb, 2, scalar_bytes(h->scalar), scalar_bytes(h->scalar)};
+  const size_t eb[4] = {sb, fm_bytes(h->scalar), scalar_bytes(h->scalar), scalar_bytes(h->scalar)};
   void *dev[4] = {nullptr, nullptr, nullptr, nullptr};
   for (int k = 0; k < 4; ++k) {
     if (!host[k]) continue;

@@ -84,6 +84,10 @@ void design_lut(IqbbDesign &d);
 void design_kernel(IqbbDesign &d);
 void design_lut_increment(IqbbDesign &d, double nco_Fs);
 void design_kernel_real(IqbbDesign &d, double Ff, double width, double Fs);   // BaseBand<int16_t>, 2^16 scaled
+// folded float path, in double and rounded to float: A(a), 128 complex entries (1 when !nco, conjugated when neg),
+// and U(r, e) = sum_{j=0}^{L-1-e} B(r, j) k[L-1-e-j] for e < n_e, 256 rows of n_e complex entries (design.cc)
+void fold_table_a(const IqbbDesign &d, bool nco, bool neg, float *A);
+void fold_table_u(const IqbbDesign &d, size_t n_e, float *U);
 
 // Window grid in closed form (SURVEY.md 8 a1).  With c = samples consumed since config(), global
 // sample n carries the window counter q(n) = max(n,1)-1 (window 0 holds ss+1 samples because

@@ -12,6 +12,7 @@
 
 #include <cmath>
 #include <complex>
+#include <vector>
 
 namespace sdrg {
 
@@ -62,6 +63,39 @@ void design_kernel(IqbbDesign &d) {
     d.k_im[i] = int32_t(q.imag());
     d.kd_re[i] = a[i].real() / norm;
     d.kd_im[i] = a[i].imag() / norm;
+  }
+}
+
+// Tables of the folded float path (iqbb_fold_kernels.cu): the 15-bit NCO phase phi = 256 a + r factorises the LUT
+// value at phi + d*inc into A(a) B(r, d).
+void fold_table_a(const IqbbDesign &d, bool nco, bool neg, float *A) {
+  for (size_t a = 0; a < 128; ++a) {
+    A[2 * a] = nco ? (float)d.lutd_re[a] : 1.0f;
+    A[2 * a + 1] = nco ? (float)(neg ? -d.lutd_im[a] : d.lutd_im[a]) : 0.0f;
+  }
+}
+
+void fold_table_u(const IqbbDesign &d, size_t n_e, float *U) {
+  const size_t L = d.order;
+  const bool nco = d.lut_inc != 0, neg = d.negative;
+  const uint64_t inc = d.lut_inc & 0x7fffu;
+  std::vector<double> br(L), bi(L);
+  for (size_t r = 0; r < 256; ++r) {
+    for (size_t j = 0; j < L; ++j) {           // B(r, j)
+      if (!nco) { br[j] = 1.0; bi[j] = 0.0; continue; }
+      const uint64_t s = (r + j * inc) >> 8;
+      const size_t idx = neg ? (size_t)((127 + 128 - (s % 128)) % 128) : (size_t)(s % 128);
+      br[j] = d.lutd_re[idx]; bi[j] = d.lutd_im[idx];
+    }
+    for (size_t e = 0; e < n_e; ++e) {
+      double sr = 0, si = 0;
+      for (size_t j = 0; j + e < L; ++j) {
+        const double kr = d.kd_re[L - 1 - e - j], ki = d.kd_im[L - 1 - e - j];
+        sr += br[j] * kr - bi[j] * ki;
+        si += br[j] * ki + bi[j] * kr;
+      }
+      U[2 * (r * n_e + e)] = (float)sr; U[2 * (r * n_e + e) + 1] = (float)si;
+    }
   }
 }
 

@@ -97,8 +97,9 @@ struct IqbbFinalizeArgs {
 struct BankAccumArgs {
   const void     *x, *hist_in;
   void           *hist_out;
-  const void     *taps;       // channels x taps_len int4 (Gauss form)
-  const void     *lut;        // 128 x int2 (shared by all channels)
+  const void     *taps;       // int: channels x taps_len int4 (Gauss form); float: taps_len x (channels rounded up to 32) float2
+  const void     *lut;        // 128 x int2 / float2 (shared by all channels)
+  const void     *tab_u;      // float: U_c(r, 0) per group of 32 channels, [group][r][channel in group] float2
   const uint32_t *inc;        // per channel: lut_inc (0 = mixer bypassed)
   const uint32_t *neg;        // per channel: negative shift
   void           *acc_cur, *acc_next;   // channels x acc_stride accumulators (int2)

@@ -70,7 +70,7 @@ int ensure_timeout_flag() {
 
 size_t elem_bytes(int scalar, int k) {   // k: 0 bb, 1 fm, 2 am, 3 usb
   const size_t s = scalar_bytes(scalar);
-  return k == 0 ? 2 * s : (k == 1 ? 2 : s);
+  return k == 0 ? 2 * s : (k == 1 ? (scalar == SDRG_T_F32 ? 4 : 2) : s);   // FM: int16, or float for a float bank
 }
 
 int grow(void **p, size_t *cap, size_t need) {

@@ -460,7 +460,8 @@ class FilterNode:
 
 class ChannelBank:
     """C independent IQBaseBand<Scalar>(Fc[c], Ff[c], width, order, sub_sample, oFs) nodes on one input
-    stream, each with FM/AM/USB demodulators connected out of place (sdrg_bank_*)."""
+    stream, each with FM/AM/USB demodulators connected out of place (sdrg_bank_*).  Scalar "s8" / "s16"
+    (bit-exact), or "f32": complex float input, float outputs (FM float32, as fm_out_dtype)."""
 
     _in_shape = (-1, 2)
     _prefix = "sdrg_bank"
@@ -498,7 +499,7 @@ class ChannelBank:
 
     def channel_info(self, c):
         inf = _lib.IqbbInfo()
-        k = np.zeros((1024, 2), dtype=np.int32)
+        k = np.zeros((1024, 2), dtype=np.float32 if self.scalar == T_F32 else np.int32)
         _lib.call("sdrg_bank_get_info", self._h, None, None, int(c), C.byref(inf), _np_ptr(k))
         return inf, k[:inf.order]
 
@@ -513,8 +514,9 @@ class ChannelBank:
         res = {} if out is None else out
         if _is_torch(x):
             import torch
-            tdt = {np.int16: torch.int16, np.int8: torch.int8}[self.dtype]
-            shapes = {"bb": ((self.channels, stride, 2), tdt), "fm": ((self.channels, stride), torch.int16),
+            tdt = {np.int16: torch.int16, np.int8: torch.int8, np.float32: torch.float32}[self.dtype]
+            fdt = {np.int16: torch.int16, np.float32: torch.float32}[fm_out_dtype(self.scalar)]
+            shapes = {"bb": ((self.channels, stride, 2), tdt), "fm": ((self.channels, stride), fdt),
                       "am": ((self.channels, stride), tdt), "usb": ((self.channels, stride), tdt)}
             for k in want:
                 if k not in res:
@@ -525,7 +527,7 @@ class ChannelBank:
                       ptr("am"), ptr("usb"), stride, C.byref(got), _stream_ptr())
             return {k: res[k][:, :got.value] for k in want}
         x = np.ascontiguousarray(x, dtype=self.dtype).reshape(-1, 2)
-        shapes = {"bb": ((self.channels, stride, 2), self.dtype), "fm": ((self.channels, stride), np.int16),
+        shapes = {"bb": ((self.channels, stride, 2), self.dtype), "fm": ((self.channels, stride), fm_out_dtype(self.scalar)),
                   "am": ((self.channels, stride), self.dtype), "usb": ((self.channels, stride), self.dtype)}
         for k in want:
             if k not in res:
@@ -553,7 +555,8 @@ ChannelBank.process_into = _bank_process_into
 class ShardedChannelBank(ChannelBank):
     """The same bank with its channels sharded by contiguous ranges over the GPUs `devices` of THIS process
     (sdrg_bank_sharded_*): torch tensors in / out live on devices[0]; numpy arrays go through every device's
-    own host<->device copies.  Bit-identical to ChannelBank."""
+    own host<->device copies.  Bit-identical to ChannelBank for "s8" / "s16"; for "f32" equal to it to float
+    rounding (window sums are float atomics)."""
 
     _prefix = "sdrg_bank_sharded"
 
