@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libsdrg.so")
 EXPERIMENTS = os.environ.get("SDRG_EXPERIMENTS", "0") not in ("", "0")     # probes / ablations / tuning switches: not shipped
-SOURCES = ["api.cu", "design.cc", "iqbb_kernels.cu", "iqbb_warp_kernels.cu", "iqbb_fold_kernels.cu", "iqbb_fold_perwin.cu"] + (["iqbb_fold_experimental.cu"] if EXPERIMENTS else []) + ["demod_kernels.cu",
+SOURCES = ["api.cu", "launch.cu", "design.cc", "iqbb_kernels.cu", "iqbb_warp_kernels.cu", "iqbb_fold_kernels.cu", "iqbb_fold_perwin.cu"] + (["iqbb_fold_experimental.cu"] if EXPERIMENTS else []) + ["demod_kernels.cu",
            "fft_kernels.cu", "fft8k_kernels.cu", "conv8k_kernels.cu", "fft_general.cu", "fft_api.cu", "bank_kernels.cu", "bank_api.cu", "multi_gpu.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-O3,-fwrapv,-fno-fast-math", "-shared", "-cudart", "static"] + (["-DSDRG_EXPERIMENTS"] if EXPERIMENTS else [])

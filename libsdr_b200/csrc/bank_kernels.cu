@@ -293,21 +293,13 @@ int launch_bank_fixed(const BankAccumArgs &a, dim3 grid, cudaStream_t st) {
   constexpr int NV = (LP + 7 + 3) / 4;
   constexpr int n_xs = kTile + 4 * NV + 8;
   const size_t smem = sizeof(uint32_t) * ((n_xs + 3) & ~3) + sizeof(int4) * (size_t)a.group * LP + sizeof(int2) * 128;
-  if (smem > 48 * 1024) SDRG_CUDA(cudaFuncSetAttribute(bank_accum_fixed_kernel<LP, IS_S8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  bank_accum_fixed_kernel<LP, IS_S8><<<grid, kT, smem, st>>>(a);
-  SDRG_CHECK_LAUNCH("bank_accum_fixed_kernel");
-  return SDRG_OK;
+  return launch("bank_accum_fixed_kernel", bank_accum_fixed_kernel<LP, IS_S8>, grid, kT, smem, st, a);
 }
 
 template <bool IS_S8>
 int dispatch_bank_fixed(int lp, const BankAccumArgs &a, dim3 grid, cudaStream_t st) {
-  switch (lp) {
-#define SDRG_CASE(N) case N: return launch_bank_fixed<N, IS_S8>(a, grid, st);
-    SDRG_CASE(2) SDRG_CASE(4) SDRG_CASE(6) SDRG_CASE(8) SDRG_CASE(10) SDRG_CASE(12) SDRG_CASE(14) SDRG_CASE(16)
-    SDRG_CASE(18) SDRG_CASE(20) SDRG_CASE(22) SDRG_CASE(24) SDRG_CASE(26) SDRG_CASE(28) SDRG_CASE(30) SDRG_CASE(32)
-#undef SDRG_CASE
-  }
-  return set_error(SDRG_ERR_RUNTIME, "no fixed-tap bank kernel for %d taps", lp);
+  return dispatch(lp, int_range<2, 32, 2>{}, [&](auto LP) { return launch_bank_fixed<LP, IS_S8>(a, grid, st); },
+                  [&] { return set_error(SDRG_ERR_RUNTIME, "no fixed-tap bank kernel for %d taps", lp); });
 }
 
 // ---- float bank: the folded weights, one channel per lane ----------------------------------------------
@@ -484,17 +476,9 @@ __global__ void __launch_bounds__(kT, 2) bank_fold_f32_kernel(const BankAccumArg
 }
 
 int launch_bank_fold_f32(const BankAccumArgs &a, cudaStream_t st) {
-  static std::atomic<int> attr_set[kMaxDevices];
-  const int dev = current_device();
-  if (!attr_set[dev]) {
-    SDRG_CUDA(cudaFuncSetAttribute(bank_fold_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kFbSmem));
-    attr_set[dev] = 1;
-  }
   const uint64_t groups = (a.channels + 31) / 32, spans = ((uint64_t)a.n + kFbSpan - 1) / kFbSpan;
   if (groups * spans > 0x7fffffffull) return set_error(SDRG_ERR_RUNTIME, "bank: too many channels x samples in one call");
-  bank_fold_f32_kernel<<<(unsigned)(groups * spans), kT, kFbSmem, st>>>(a);
-  SDRG_CHECK_LAUNCH("bank_fold_f32_kernel");
-  return SDRG_OK;
+  return launch("bank_fold_f32_kernel", bank_fold_f32_kernel, (unsigned)(groups * spans), kT, kFbSmem, st, a);
 }
 
 // finalize for every channel: blockIdx.y = channel
@@ -527,29 +511,16 @@ int launch_bank_accum(int scalar, const BankAccumArgs &a, cudaStream_t st) {
     const int lp = (int)((a.taps_len + 1) & ~1u);
     return scalar == SDRG_T_S8 ? dispatch_bank_fixed<true>(lp, a, grid, st) : dispatch_bank_fixed<false>(lp, a, grid, st);
   }
-  if (scalar == SDRG_T_S8) {
-    if (smem > 48 * 1024) SDRG_CUDA(cudaFuncSetAttribute(bank_accum_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    bank_accum_kernel<true><<<grid, kT, smem, st>>>(a);
-  } else {
-    if (smem > 48 * 1024) SDRG_CUDA(cudaFuncSetAttribute(bank_accum_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    bank_accum_kernel<false><<<grid, kT, smem, st>>>(a);
-  }
-  SDRG_CHECK_LAUNCH("bank_accum_kernel");
-  return SDRG_OK;
+  return launch("bank_accum_kernel", scalar == SDRG_T_S8 ? bank_accum_kernel<true> : bank_accum_kernel<false>, grid, kT, smem, st, a);
 }
 
 int launch_bank_finalize(int scalar, const IqbbFinalizeArgs &a, const BankFinalizeStrides &s, uint32_t channels, cudaStream_t st) {
   if (channels == 0) return SDRG_OK;
   const unsigned gx = (a.n_out + 255) / 256;
   dim3 grid(gx ? gx : 1, channels);
-  switch (scalar) {
-    case SDRG_T_S8: bank_finalize_kernel<SDRG_T_S8><<<grid, 256, 0, st>>>(a, s); break;
-    case SDRG_T_S16: bank_finalize_kernel<SDRG_T_S16><<<grid, 256, 0, st>>>(a, s); break;
-    case SDRG_T_F32: bank_finalize_kernel<SDRG_T_F32><<<grid, 256, 0, st>>>(a, s); break;
-    default: return set_error(SDRG_ERR_RUNTIME, "bank: no finalize kernel for scalar %d", scalar);
-  }
-  SDRG_CHECK_LAUNCH("bank_finalize_kernel");
-  return SDRG_OK;
+  return dispatch(scalar, std::integer_sequence<int, SDRG_T_S8, SDRG_T_S16, SDRG_T_F32>{},
+                  [&](auto S) { return launch("bank_finalize_kernel", bank_finalize_kernel<S>, grid, 256, 0, st, a, s); },
+                  [&] { return set_error(SDRG_ERR_RUNTIME, "bank: no finalize kernel for scalar %d", scalar); });
 }
 
 }  // namespace sdrg

@@ -41,11 +41,6 @@ static inline int env_int(const char *name, int dflt) { const char *e = getenv(n
 static inline int env_int(const char *, int dflt) { return dflt; }
 #endif
 
-// Per-device one-time launch setup.  Function attributes (dynamic shared memory opt-in) and
-// occupancy are properties of (kernel, device): cache them per device, not per process.
-constexpr int kMaxDevices = 64;
-static inline int current_device() { int d = 0; cudaGetDevice(&d); return (d >= 0 && d < kMaxDevices) ? d : 0; }
-
 // ---- scalar helpers ---------------------------------------------------------------------------
 static inline size_t scalar_bytes(int scalar) {
   switch (scalar) {

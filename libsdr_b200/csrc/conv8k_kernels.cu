@@ -142,35 +142,18 @@ __global__ void __launch_bounds__(kT, 2) conv8k_kernel(const FilterArgs a, const
 
 }  // namespace
 
-int conv8k_grid(size_t n_blocks) {      // CTAs launch_conv8k will use (the bank's scratch is 64 KB per CTA)
-  const int dev = current_device();
-  static std::atomic<int> attr[kMaxDevices];
-  if (!attr[dev]) {
-    if (cudaFuncSetAttribute(conv8k_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes) != cudaSuccess ||
-        cudaFuncSetAttribute(conv8k_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes) != cudaSuccess) {
-      cudaGetLastError();
-      return 0;
-    }
-    attr[dev] = 1;
-  }
-  static std::atomic<int> res[kMaxDevices];
-  const int resident = resident_ctas((const void *)conv8k_kernel<true>, dev, res);
-  return (int)(n_blocks < (size_t)resident ? n_blocks : (size_t)resident);
+int conv8k_grid(size_t n_blocks, int *grid) {      // CTAs launch_conv8k will use (the bank's scratch is 64 KB per CTA)
+  int resident = 0;
+  const int rc = kernel_setup((const void *)conv8k_kernel<true>, kT, kSmemBytes, &resident);
+  *grid = (int)(n_blocks < (size_t)resident ? n_blocks : (size_t)resident);
+  return rc;
 }
 
 int launch_conv8k(const FilterArgs &a, size_t n_blocks, cudaStream_t st) {
   if (n_blocks == 0) return SDRG_OK;
   if (n_blocks > 0x7fffffffull) return set_error(SDRG_ERR_ARG, "FilterNode: too many blocks in one call");
-  const int grid = conv8k_grid(n_blocks);
-  if (grid <= 0) return set_error(SDRG_ERR_CUDA, "FilterNode: cannot configure the block-4096 kernel");
-  if (a.n_filters > 1) {
-    if (!a.spec) return set_error(SDRG_ERR_RUNTIME, "FilterNode: the filter bank needs its spectrum scratch");
-    conv8k_kernel<true><<<grid, kT, kSmemBytes, st>>>(a, (int)n_blocks);
-  } else {
-    conv8k_kernel<false><<<grid, kT, kSmemBytes, st>>>(a, (int)n_blocks);
-  }
-  SDRG_CHECK_LAUNCH("conv8k_kernel");
-  return SDRG_OK;
+  if (a.n_filters > 1 && !a.spec) return set_error(SDRG_ERR_RUNTIME, "FilterNode: the filter bank needs its spectrum scratch");
+  return launch_persistent("conv8k_kernel", a.n_filters > 1 ? conv8k_kernel<true> : conv8k_kernel<false>, n_blocks, kT, kSmemBytes, st, a, (int)n_blocks);
 }
 
 }  // namespace sdrg

@@ -3,6 +3,7 @@
 // These are HBM-streaming elementwise kernels: 4 (2, 8) bytes in and 2 (1, 4) bytes out per
 // sample, one sample per thread-iteration, grid-stride, coalesced.
 #include "iqbb_kernels.cuh"
+#include "launch.cuh"
 #include "demod_math.cuh"
 
 namespace sdrg {
@@ -179,16 +180,8 @@ __global__ void __launch_bounds__(256) autocast_kernel(const void *__restrict__ 
 
 int launch_autocast(int kind, const void *in, size_t n_scalars, void *out, cudaStream_t st) {
   if (n_scalars == 0) return SDRG_OK;
-  const unsigned g = grid_for(n_scalars);
-  switch (kind) {
-#define SDRG_CASE(K) case K: autocast_kernel<K><<<g, 256, 0, st>>>(in, n_scalars, out); break;
-    SDRG_CASE(1) SDRG_CASE(2) SDRG_CASE(3) SDRG_CASE(4) SDRG_CASE(5) SDRG_CASE(6) SDRG_CASE(7)
-    SDRG_CASE(8) SDRG_CASE(9) SDRG_CASE(10) SDRG_CASE(11) SDRG_CASE(12) SDRG_CASE(13) SDRG_CASE(14)
-#undef SDRG_CASE
-    default: return set_error(SDRG_ERR_ARG, "AutoCast: unknown cast kind %d", kind);
-  }
-  SDRG_CHECK_LAUNCH("autocast_kernel");
-  return SDRG_OK;
+  return dispatch(kind, int_range<1, 14>{}, [&](auto K) { return launch("autocast_kernel", autocast_kernel<K>, grid_for(n_scalars), 256, 0, st, in, n_scalars, out); },
+                  [&] { return set_error(SDRG_ERR_ARG, "AutoCast: unknown cast kind %d", kind); });
 }
 
 int launch_fmdeemph(const void *in, void *out, size_t n, size_t streams, size_t stride, int alpha, void *avg, cudaStream_t st) {

@@ -118,29 +118,10 @@ void fft8k_permute_kernel(const float *kern, float *kperm) {
 int launch_fft8k(const void *in, void *out, int n, int inverse, size_t batch, const void *tab, cudaStream_t st) {
   if (batch == 0) return SDRG_OK;
   if (batch > 0x7fffffffull) return set_error(SDRG_ERR_ARG, "FFT plan: batch too large");
-  const int dev = current_device();
-  static std::atomic<int> attr[kMaxDevices];
-  if (!attr[dev]) {
-    SDRG_CUDA(cudaFuncSetAttribute(fft8k_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
-    SDRG_CUDA(cudaFuncSetAttribute(fft8k_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
-    SDRG_CUDA(cudaFuncSetAttribute(fft8k_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
-    SDRG_CUDA(cudaFuncSetAttribute(fft8k_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
-    attr[dev] = 1;
-  }
-  static std::atomic<int> res[kMaxDevices];
-  const int resident = resident_ctas((const void *)fft8k_kernel<false, true>, dev, res);
-  const size_t items = n == 8192 ? batch : (batch + 1) / 2;
-  const unsigned grid = (unsigned)(items < (size_t)resident ? items : (size_t)resident);
-  const float2 *i2 = (const float2 *)in; float2 *o2 = (float2 *)out; const float2 *t2 = (const float2 *)tab;
-  if (n == 8192) {
-    if (inverse) fft8k_kernel<true, true><<<grid, kT, kSmemBytes, st>>>(i2, o2, (int)batch, t2);
-    else fft8k_kernel<false, true><<<grid, kT, kSmemBytes, st>>>(i2, o2, (int)batch, t2);
-  } else {
-    if (inverse) fft8k_kernel<true, false><<<grid, kT, kSmemBytes, st>>>(i2, o2, (int)batch, t2);
-    else fft8k_kernel<false, false><<<grid, kT, kSmemBytes, st>>>(i2, o2, (int)batch, t2);
-  }
-  SDRG_CHECK_LAUNCH("fft8k_kernel");
-  return SDRG_OK;
+  const bool full = n == 8192;
+  auto *kern = inverse ? (full ? fft8k_kernel<true, true> : fft8k_kernel<true, false>) : (full ? fft8k_kernel<false, true> : fft8k_kernel<false, false>);
+  return launch_persistent("fft8k_kernel", kern, full ? batch : (batch + 1) / 2, kT, kSmemBytes, st,
+                           (const float2 *)in, (float2 *)out, (int)batch, (const float2 *)tab);
 }
 
 }  // namespace sdrg

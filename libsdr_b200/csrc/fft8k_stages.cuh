@@ -4,8 +4,8 @@
 #pragma once
 #include "fft_kernels.cuh"
 #include "fft_device.cuh"
+#include "launch.cuh"
 
-#include <atomic>
 #include <cmath>
 #include <vector>
 
@@ -107,16 +107,6 @@ __device__ __forceinline__ void store16(const float2 *v, float2 *H, const int p0
   float4 *h4 = (float4 *)(H + p0);
 #pragma unroll
   for (int k = 0; k < 8; ++k) h4[k] = make_float4(v[2 * k].x, v[2 * k].y, v[2 * k + 1].x, v[2 * k + 1].y);
-}
-
-int resident_ctas(const void *fn, int dev, std::atomic<int> *cache) {
-  if (!cache[dev]) {
-    int sms = 0, per_sm = 0;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kT, kSmemBytes);
-    cache[dev] = sms * (per_sm > 0 ? per_sm : 1);
-  }
-  return cache[dev];
 }
 
 

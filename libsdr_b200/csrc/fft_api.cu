@@ -411,7 +411,12 @@ int sdrg_filter_process_dev(sdrg_filter *h, const void *d_in, size_t n_in, void 
     a.block = (int)N; a.log2n = h->log2n; a.n_filters = (int)h->bands.size();
     a.spec = nullptr; a.kperm = h->d_kperm; a.tab8k = h->d_tab8k;
     size_t spec_bytes = nblk * 2 * N * sb;
-    if (a.n_filters > 1 && 2 * N == 8192 && a.kperm) spec_bytes = (size_t)conv8k_grid(nblk) * 8192 * sb;   // one 64 KB line per CTA
+    if (a.n_filters > 1 && 2 * N == 8192 && a.kperm) {      // one 64 KB line per CTA
+      int grid = 0;
+      rc = conv8k_grid(nblk, &grid);
+      if (rc) return rc;
+      spec_bytes = (size_t)grid * 8192 * sb;
+    }
     if (a.n_filters > 1 && 2 * N >= 512 && spec_bytes <= ((size_t)2 << 30)) {
       rc = grow_dev(&h->d_spec, &h->spec_cap, spec_bytes);
       if (rc) return rc;

@@ -20,7 +20,7 @@
 // in double on the host.  Data ping-pongs between shared-memory buffers; one __syncthreads per stage.
 #include "fft_kernels.cuh"
 #include "fft_device.cuh"
-#include <atomic>
+#include "launch.cuh"
 #include <cstdlib>
 
 namespace sdrg {
@@ -366,72 +366,30 @@ int launch_fft_batch(const void *in, void *out, int n, int log2n, int inverse, s
   if (r16 && n >= 256 && batch <= 0x7fffffffull) {
     const int tpf = n / 16, fpc = tpf >= 256 ? 1 : 256 / tpf;
     const size_t smem = (size_t)fpc * padded_len(n) * sizeof(float2);
-    static std::atomic<size_t> attr16[kMaxDevices];
-    const int dev = current_device();
-    if (smem > 48 * 1024 && smem > attr16[dev]) {
-      SDRG_CUDA(cudaFuncSetAttribute(fft_batch_r16_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      SDRG_CUDA(cudaFuncSetAttribute(fft_batch_r16_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      attr16[dev] = smem;
-    }
-    const unsigned grid = (unsigned)((batch + fpc - 1) / fpc);
-    if (inverse) fft_batch_r16_kernel<true><<<grid, tpf * fpc, smem, st>>>((const float2 *)in, (float2 *)out, n, log2n, (int)batch, (const float2 *)tw);
-    else fft_batch_r16_kernel<false><<<grid, tpf * fpc, smem, st>>>((const float2 *)in, (float2 *)out, n, log2n, (int)batch, (const float2 *)tw);
-    SDRG_CHECK_LAUNCH("fft_batch_r16_kernel");
-    return SDRG_OK;
-  }
-  const size_t smem = (size_t)2 * padded_len(n) * sizeof(float2);
-  static std::atomic<size_t> attr[kMaxDevices];
-  const int dev = current_device();
-  if (smem > 48 * 1024 && smem > attr[dev]) {
-    SDRG_CUDA(cudaFuncSetAttribute(fft_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr[dev] = smem;
+    return launch("fft_batch_r16_kernel", inverse ? fft_batch_r16_kernel<true> : fft_batch_r16_kernel<false>, (unsigned)((batch + fpc - 1) / fpc),
+                  tpf * fpc, smem, st, (const float2 *)in, (float2 *)out, n, log2n, (int)batch, (const float2 *)tw);
   }
   int threads = n / 8; if (threads < 32) threads = 32; if (threads > 1024) threads = 1024;
-  fft_batch_kernel<<<(unsigned)batch, threads, smem, st>>>((const float2 *)in, (float2 *)out, n, log2n, inverse, (const float2 *)tw);
-  SDRG_CHECK_LAUNCH("fft_batch_kernel");
-  return SDRG_OK;
+  return launch("fft_batch_kernel", fft_batch_kernel, (unsigned)batch, threads, (size_t)2 * padded_len(n) * sizeof(float2), st,
+                (const float2 *)in, (float2 *)out, n, log2n, inverse, (const float2 *)tw);
 }
 
 int launch_filter_ola(const FilterArgs &a, size_t n_blocks, cudaStream_t st) {
   if (n_blocks == 0) return SDRG_OK;
   const int n = 2 * a.block;
   if (n == 8192 && a.n_filters >= 1 && a.kperm && a.tab8k) return launch_conv8k(a, n_blocks, st);
-  const size_t smem = (size_t)3 * padded_len(n) * sizeof(float2);
-  static std::atomic<size_t> attr[kMaxDevices];
-  const int dev = current_device();
-  if (smem > 48 * 1024 && smem > attr[dev]) {
-    SDRG_CUDA(cudaFuncSetAttribute(filter_ola_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr[dev] = smem;
-  }
-  int threads = n / 8; if (threads < 32) threads = 32; if (threads > 1024) threads = 1024;
   static const int r16 = env_int("SDRG_FFT_R16", 1);
   if (n >= 512 && (a.n_filters == 1 || (r16 && a.spec))) {   // in-place stages on a single buffer (n == 16 * threads)
     const size_t smem1 = (size_t)padded_len(n) * sizeof(float2);
-    static std::atomic<size_t> attr1[kMaxDevices];
-    if (smem1 > 48 * 1024 && smem1 > attr1[dev]) {
-      SDRG_CUDA(cudaFuncSetAttribute(filter_ola1_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-      SDRG_CUDA(cudaFuncSetAttribute(filter_ola1_r16_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-      SDRG_CUDA(cudaFuncSetAttribute(filter_ola1_r16_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-      SDRG_CUDA(cudaFuncSetAttribute(filter_ola1_r16_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
-      attr1[dev] = smem1;
-    }
-    if (!r16) {
-      filter_ola1_kernel<<<(unsigned)n_blocks, n / 16, smem1, st>>>(a);
-      SDRG_CHECK_LAUNCH("filter_ola1_kernel");
-    } else if (a.n_filters == 1) {
-      filter_ola1_r16_kernel<0><<<(unsigned)n_blocks, n / 16, smem1, st>>>(a);
-      SDRG_CHECK_LAUNCH("filter_ola1_r16_kernel");
-    } else {                                    // bank: one forward pass, then every (block, filter) pair on its own CTA
-      filter_ola1_r16_kernel<1><<<(unsigned)n_blocks, n / 16, smem1, st>>>(a);
-      SDRG_CHECK_LAUNCH("filter_ola1_r16_kernel<fwd>");
-      filter_ola1_r16_kernel<2><<<dim3((unsigned)n_blocks, (unsigned)a.n_filters), n / 16, smem1, st>>>(a);
-      SDRG_CHECK_LAUNCH("filter_ola1_r16_kernel<inv>");
-    }
-    return SDRG_OK;
+    if (!r16) return launch("filter_ola1_kernel", filter_ola1_kernel, (unsigned)n_blocks, n / 16, smem1, st, a);
+    if (a.n_filters == 1) return launch("filter_ola1_r16_kernel", filter_ola1_r16_kernel<0>, (unsigned)n_blocks, n / 16, smem1, st, a);
+    // bank: one forward pass, then every (block, filter) pair on its own CTA
+    const int rc = launch("filter_ola1_r16_kernel<fwd>", filter_ola1_r16_kernel<1>, (unsigned)n_blocks, n / 16, smem1, st, a);
+    if (rc) return rc;
+    return launch("filter_ola1_r16_kernel<inv>", filter_ola1_r16_kernel<2>, dim3((unsigned)n_blocks, (unsigned)a.n_filters), n / 16, smem1, st, a);
   }
-  filter_ola_kernel<<<(unsigned)n_blocks, threads, smem, st>>>(a);
-  SDRG_CHECK_LAUNCH("filter_ola_kernel");
-  return SDRG_OK;
+  int threads = n / 8; if (threads < 32) threads = 32; if (threads > 1024) threads = 1024;
+  return launch("filter_ola_kernel", filter_ola_kernel, (unsigned)n_blocks, threads, (size_t)3 * padded_len(n) * sizeof(float2), st, a);
 }
 
 }  // namespace sdrg

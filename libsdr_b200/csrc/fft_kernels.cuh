@@ -33,7 +33,7 @@ void fft8k_tables(std::vector<float> &tab);                           // host: t
 void fft8k_permute_kernel(const float *kern_8192, float *kperm_8192); // host: spectrum -> kernel order, x 1/8192
 int launch_fft8k(const void *in, void *out, int n, int inverse, size_t batch, const void *tab, cudaStream_t st);
 int launch_conv8k(const FilterArgs &a, size_t n_blocks, cudaStream_t st);
-int conv8k_grid(size_t n_blocks);   // CTAs that launch will use: a filter bank needs 64 KB of FilterArgs::spec per CTA
+int conv8k_grid(size_t n_blocks, int *grid);   // CTAs that launch will use: a filter bank needs 64 KB of FilterArgs::spec per CTA
 
 
 // fft_general.cu: every other size, composed from the kernels above (see its header comment)

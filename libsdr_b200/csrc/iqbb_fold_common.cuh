@@ -2,7 +2,7 @@
 // experimental / instrumentation variants (iqbb_fold_experimental.cu).  See iqbb_fold_kernels.cu for the method.
 #pragma once
 #include "iqbb_kernels.cuh"
-#include <atomic>
+#include "launch.cuh"
 #include <cstdlib>
 
 namespace sdrg {

@@ -266,30 +266,23 @@ __global__ void __launch_bounds__(kFoldThreads, MODE == 1 ? 4 : 3) iqbb_fold_pro
 template <int MODE>
 int launch_fold_probe_t(IqbbFoldArgs a, cudaStream_t st) {
   const size_t smem = (size_t)kFoldWarps * kStageRows * kStagePitch * sizeof(float2);
-  int sms = 0, per_sm = 0;
-  const int dev = current_device();
-  SDRG_CUDA(cudaFuncSetAttribute(iqbb_fold_probe_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  SDRG_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  SDRG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, iqbb_fold_probe_kernel<MODE>, kFoldThreads, smem));
-  static const int cap = [] { const char *e = getenv("SDRG_FOLD_PROBE_CTAS"); return e ? atoi(e) : 0; }();
-  if (cap > 0 && cap < per_sm) per_sm = cap;
-  const uint64_t resident = (uint64_t)sms * (per_sm > 0 ? per_sm : 1);
+  int resident = 0;
+  const int rc = kernel_setup((const void *)iqbb_fold_probe_kernel<MODE>, kFoldThreads, smem, &resident);
+  if (rc) return rc;
+  static const int cap = [] { const char *e = getenv("SDRG_FOLD_PROBE_CTAS"); return e ? atoi(e) : 0; }();   // CTAs per SM
+  if (cap > 0) {
+    int dev = 0, sms = 0;
+    SDRG_CUDA(cudaGetDevice(&dev));
+    SDRG_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    resident = std::min(resident, sms * cap);
+  }
   const uint64_t want = ((uint64_t)a.n_chunks + kFoldWarps - 1) / kFoldWarps;
-  iqbb_fold_probe_kernel<MODE><<<(unsigned)(want < resident ? want : resident), kFoldThreads, smem, st>>>(a);
-  SDRG_CHECK_LAUNCH("iqbb_fold_probe_kernel");
-  return SDRG_OK;
+  return launch("iqbb_fold_probe_kernel", iqbb_fold_probe_kernel<MODE>, (unsigned)std::min<uint64_t>(want, resident), kFoldThreads, smem, st, a);
 }
 
 }  // namespace
 
 int launch_fold_tma(IqbbFoldArgs a, cudaStream_t st) {
-  static std::atomic<bool> attr_set[kMaxDevices];
-  const size_t smem = (size_t)kFoldWarps * kTmaRing * sizeof(float2);
-  const int dev = current_device();
-  if (!attr_set[dev]) {
-    SDRG_CUDA(cudaFuncSetAttribute(iqbb_fold_f32_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_set[dev] = true;
-  }
   // one contiguous 2 KB-aligned segment per warp; ~2 waves of 148 x 3 CTAs
   const uint64_t target_warps = 148ull * 3 * kFoldWarps * 2;
   uint64_t seg = (a.n + target_warps - 1) / target_warps;
@@ -297,10 +290,8 @@ int launch_fold_tma(IqbbFoldArgs a, cudaStream_t st) {
   if (seg < (uint64_t)kTmaTile) seg = kTmaTile;
   a.seg = (uint32_t)seg;
   const uint64_t per_block = seg * kFoldWarps;
-  const unsigned grid = (unsigned)((a.n + per_block - 1) / per_block);
-  iqbb_fold_f32_tma_kernel<<<grid, kFoldThreads, smem, st>>>(a);
-  SDRG_CHECK_LAUNCH("iqbb_fold_f32_tma_kernel");
-  return SDRG_OK;
+  return launch("iqbb_fold_f32_tma_kernel", iqbb_fold_f32_tma_kernel, (unsigned)((a.n + per_block - 1) / per_block), kFoldThreads,
+                (size_t)kFoldWarps * kTmaRing * sizeof(float2), st, a);
 }
 
 

@@ -244,58 +244,24 @@ __global__ void __launch_bounds__(kFoldThreads, S <= 8 ? 4 : (S <= 13 ? 3 : 2)) 
 
 template <int S, int P = 0, int TS = 3>
 static int launch_fold_win_s(const IqbbFoldArgs &a, cudaStream_t st) {
-  static std::atomic<int> resident_dev[kMaxDevices];
   const size_t smem = (size_t)kFoldWarps * kStageRows * kStagePitch * sizeof(float2);
-  const int dev = current_device();
-  if (!resident_dev[dev]) {
-    SDRG_CUDA(cudaFuncSetAttribute(iqbb_fold_f32_win_kernel<S, P, TS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int sms = 0, per_sm = 0;
-    SDRG_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    SDRG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, iqbb_fold_f32_win_kernel<S, P, TS>, kFoldThreads, smem));
-    resident_dev[dev] = sms * (per_sm > 0 ? per_sm : 1);
-  }
-  const uint64_t resident = (uint64_t)resident_dev[dev];
   const uint64_t want = ((uint64_t)a.n_chunks + kFoldWarps - 1) / kFoldWarps;
-  iqbb_fold_f32_win_kernel<S, P, TS><<<(unsigned)(want < resident ? want : resident), kFoldThreads, smem, st>>>(a);
-  SDRG_CHECK_LAUNCH("iqbb_fold_f32_win_kernel");
-  return SDRG_OK;
+  return launch_persistent("iqbb_fold_f32_win_kernel", iqbb_fold_f32_win_kernel<S, P, TS>, want, kFoldThreads, smem, st, a);
 }
 
 static int launch_fold_win(const IqbbFoldArgs &a, cudaStream_t st) {
+  const int s = (int)((a.ss + 31) / 32);
 #ifdef SDRG_EXPERIMENTS
   static const int wp = env_int("SDRG_FOLD_WINP", 0);   // ablations of the S = 13 kernel: WRONG RESULTS, timing only
-  if (wp && (a.ss + 31) / 32 == 13) {
-    switch (wp) {
-      case 1: return launch_fold_win_s<13, 1>(a, st); case 2: return launch_fold_win_s<13, 2>(a, st);
-      case 3: return launch_fold_win_s<13, 3>(a, st); case 4: return launch_fold_win_s<13, 4>(a, st);
-      case 5: return launch_fold_win_s<13, 5>(a, st); case 6: return launch_fold_win_s<13, 6>(a, st);
-      case 7: return launch_fold_win_s<13, 7>(a, st); case 8: return launch_fold_win_s<13, 8>(a, st); default: break;
-    }
-  }
+  if (wp >= 1 && wp <= 8 && s == 13)
+    return dispatch(wp, int_range<1, 8>{}, [&](auto P) { return launch_fold_win_s<13, P>(a, st); }, [] { return SDRG_OK; });
 #endif
-  if (a.taps_len > 65) {      // 66..129 taps: the tail reaches back up to five ring steps (ss >= taps - 1 >= 65, so S >= 3)
-    switch ((a.ss + 31) / 32) {
-      case 3: return launch_fold_win_s<3, 0, 5>(a, st);   case 4: return launch_fold_win_s<4, 0, 5>(a, st);
-      case 5: return launch_fold_win_s<5, 0, 5>(a, st);   case 6: return launch_fold_win_s<6, 0, 5>(a, st);
-      case 7: return launch_fold_win_s<7, 0, 5>(a, st);   case 8: return launch_fold_win_s<8, 0, 5>(a, st);
-      case 9: return launch_fold_win_s<9, 0, 5>(a, st);   case 10: return launch_fold_win_s<10, 0, 5>(a, st);
-      case 11: return launch_fold_win_s<11, 0, 5>(a, st); case 12: return launch_fold_win_s<12, 0, 5>(a, st);
-      case 13: return launch_fold_win_s<13, 0, 5>(a, st); case 14: return launch_fold_win_s<14, 0, 5>(a, st);
-      case 15: return launch_fold_win_s<15, 0, 5>(a, st); case 16: return launch_fold_win_s<16, 0, 5>(a, st);
-      default: return set_error(SDRG_ERR_RUNTIME, "IQBaseBand<float>: window-pipelined kernel needs 65 <= sub_sample <= 512 for more than 65 taps");
-    }
-  }
-  switch ((a.ss + 31) / 32) {
-    case 1: return launch_fold_win_s<1>(a, st);   case 2: return launch_fold_win_s<2>(a, st);
-    case 3: return launch_fold_win_s<3>(a, st);   case 4: return launch_fold_win_s<4>(a, st);
-    case 5: return launch_fold_win_s<5>(a, st);   case 6: return launch_fold_win_s<6>(a, st);
-    case 7: return launch_fold_win_s<7>(a, st);   case 8: return launch_fold_win_s<8>(a, st);
-    case 9: return launch_fold_win_s<9>(a, st);   case 10: return launch_fold_win_s<10>(a, st);
-    case 11: return launch_fold_win_s<11>(a, st); case 12: return launch_fold_win_s<12>(a, st);
-    case 13: return launch_fold_win_s<13>(a, st); case 14: return launch_fold_win_s<14>(a, st);
-    case 15: return launch_fold_win_s<15>(a, st); case 16: return launch_fold_win_s<16>(a, st);
-    default: return set_error(SDRG_ERR_RUNTIME, "IQBaseBand<float>: window-pipelined kernel needs sub_sample <= 512");
-  }
+  if (a.taps_len > 65)        // 66..129 taps: the tail reaches back up to five ring steps (ss >= taps - 1 >= 65, so S >= 3)
+    return dispatch(s, int_range<3, 16>{}, [&](auto S) { return launch_fold_win_s<S, 0, 5>(a, st); }, [] {
+      return set_error(SDRG_ERR_RUNTIME, "IQBaseBand<float>: window-pipelined kernel needs 65 <= sub_sample <= 512 for more than 65 taps");
+    });
+  return dispatch(s, int_range<1, 16>{}, [&](auto S) { return launch_fold_win_s<S>(a, st); },
+                  [] { return set_error(SDRG_ERR_RUNTIME, "IQBaseBand<float>: window-pipelined kernel needs sub_sample <= 512"); });
 }
 
 // ---- short windows (2 <= ss < 128) ------------------------------------------------------------------
@@ -400,21 +366,8 @@ __global__ void __launch_bounds__(kFoldThreads, 4) iqbb_fold_f32_small_kernel(co
 }
 
 static int launch_fold_small(const IqbbFoldArgs &a, cudaStream_t st) {
-  static std::atomic<int> resident_dev[kMaxDevices];
-  const size_t smem = (size_t)2 * kSmallTile * sizeof(float2);
-  const int dev = current_device();
-  if (!resident_dev[dev]) {
-    SDRG_CUDA(cudaFuncSetAttribute(iqbb_fold_f32_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int sms = 0, per_sm = 0;
-    SDRG_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    SDRG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, iqbb_fold_f32_small_kernel, kFoldThreads, smem));
-    resident_dev[dev] = sms * (per_sm > 0 ? per_sm : 1);
-  }
   const uint64_t n_tiles = ((uint64_t)a.n + kSmallTile - 1) / kSmallTile;
-  const uint64_t resident = (uint64_t)resident_dev[dev];
-  iqbb_fold_f32_small_kernel<<<(unsigned)(n_tiles < resident ? n_tiles : resident), kFoldThreads, smem, st>>>(a);
-  SDRG_CHECK_LAUNCH("iqbb_fold_f32_small_kernel");
-  return SDRG_OK;
+  return launch_persistent("iqbb_fold_f32_small_kernel", iqbb_fold_f32_small_kernel, n_tiles, kFoldThreads, (size_t)2 * kSmallTile * sizeof(float2), st, a);
 }
 
 }  // namespace
@@ -459,23 +412,9 @@ static int launch_fold_ldg(IqbbFoldArgs a, cudaStream_t st, int *which) {
 #ifdef SDRG_EXPERIMENTS
   if (probe >= 1 && probe <= 3) return launch_fold_probe(probe, a, st);
 #endif
-  static std::atomic<int> resident_dev[kMaxDevices];     // CTAs that fit the device at once: SMs x occupancy
-  const size_t smem = (size_t)kFoldWarps * kStageRows * kStagePitch * sizeof(float2);
-  const int dev = current_device();
-  if (!resident_dev[dev]) {
-    SDRG_CUDA(cudaFuncSetAttribute(iqbb_fold_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int sms = 0, per_sm = 0;
-    SDRG_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    SDRG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, iqbb_fold_f32_kernel, kFoldThreads, smem));
-    resident_dev[dev] = sms * (per_sm > 0 ? per_sm : 1);
-  }
   *which = 2;
-  const int resident = resident_dev[dev];
-  const uint64_t want = (n_chunks + kFoldWarps - 1) / kFoldWarps;
-  const unsigned grid = (unsigned)(want < (uint64_t)resident ? want : (uint64_t)resident);
-  iqbb_fold_f32_kernel<<<grid, kFoldThreads, smem, st>>>(a);
-  SDRG_CHECK_LAUNCH("iqbb_fold_f32_kernel");
-  return SDRG_OK;
+  const size_t smem = (size_t)kFoldWarps * kStageRows * kStagePitch * sizeof(float2);
+  return launch_persistent("iqbb_fold_f32_kernel", iqbb_fold_f32_kernel, (n_chunks + kFoldWarps - 1) / kFoldWarps, kFoldThreads, smem, st, a);
 }
 
 int launch_iqbb_fold(const IqbbFoldArgs &a, cudaStream_t st, int *which_out) {

@@ -332,35 +332,6 @@ __global__ void __launch_bounds__(1024, 1) iqbb_fold_f32_perwin16_kernel(const I
   }
 }
 
-// occupancy depends on the dynamic shared memory size, which depends on the configuration: cached per (device, size)
-template <typename Kern>
-int perwin_launch(Kern kern, int threads, const IqbbFoldArgs &a, const PerwinGeom &geo, uint64_t want, size_t smem, cudaStream_t st,
-                  std::atomic<int> *resident_dev, std::atomic<int> *smem_for, std::atomic<int> *smem_max) {
-  const int dev = current_device();
-  if (smem_max[dev] < (int)smem) {
-    SDRG_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    smem_max[dev] = (int)smem;
-  }
-  if (smem_for[dev] != (int)smem * 8 + threads / 256 || !resident_dev[dev]) {
-    int sms = 0, per_sm = 0;
-    SDRG_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    SDRG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
-    resident_dev[dev] = sms * (per_sm > 0 ? per_sm : 1);
-    smem_for[dev] = (int)smem * 8 + threads / 256;
-  }
-  const uint64_t resident = (uint64_t)resident_dev[dev];
-  kern<<<(unsigned)(want < resident ? want : resident), threads, smem, st>>>(a, geo);
-  SDRG_CHECK_LAUNCH("iqbb_fold_f32_perwin_kernel");
-  return SDRG_OK;
-}
-
-template <int K>
-int launch_perwin16(int groups, const IqbbFoldArgs &a, const PerwinGeom &geo, size_t smem, cudaStream_t st) {
-  static std::atomic<int> resident_dev[kMaxDevices], smem_for[kMaxDevices], smem_max[kMaxDevices];
-  const uint64_t want = (geo.n_tiles + groups - 1) / groups;
-  return perwin_launch(iqbb_fold_f32_perwin16_kernel<K>, groups * kPwGroup, a, geo, want > 0 ? want : 1, smem, st, resident_dev, smem_for, smem_max);
-}
-
 static uint32_t pw1_max() { static const int v = env_int("SDRG_FOLD_PERWIN1_MAX", 22); return (uint32_t)v; }   // ss <= this: a thread per window; above: a half warp per window
 
 constexpr size_t kPwMaxSmem = 220 * 1024;
@@ -437,14 +408,13 @@ int launch_fold_perwin(const IqbbFoldArgs &a_in, cudaStream_t st) {
   const size_t table = ((size_t)a.v_rows * a.v_pitch + 1) & ~(size_t)1;
   if (a.ss <= pw1_max()) {
     // small table, several CTAs per SM with two buffers each (measured: 3 CTAs x 2 buffers beat 2 CTAs x 3)
-    static std::atomic<int> resident_dev[kMaxDevices], smem_for[kMaxDevices], smem_max[kMaxDevices];
     geo.x_tile = (uint32_t)tile_elems(a, 0, &geo.delta);
     geo.pitch = a.ss + geo.delta;
     geo.chunk = 16;
     if (geo.delta) while (geo.chunk + (geo.chunk + a.ss - 2) / a.ss > 16u) --geo.chunk;   // samples + window borders crossed <= 16 slots
     geo.n_tiles = (a.d_hi - a.d_lo + 1 + 255u) / 256u;
-    return perwin_launch(iqbb_fold_f32_perwin1_kernel, kPw1Threads, a, geo, geo.n_tiles, (table + geo.stages * (size_t)geo.x_tile) * sizeof(float2), st,
-                         resident_dev, smem_for, smem_max);
+    return launch_persistent("iqbb_fold_f32_perwin_kernel", iqbb_fold_f32_perwin1_kernel, geo.n_tiles, kPw1Threads,
+                             (table + geo.stages * (size_t)geo.x_tile) * sizeof(float2), st, a, geo);
   }
   int k = 1, groups = 1;
   shape16(a, table, &k, &groups);
@@ -453,11 +423,10 @@ int launch_fold_perwin(const IqbbFoldArgs &a_in, cudaStream_t st) {
   const size_t smem = (table + (size_t)groups * geo.stages * geo.x_tile) * sizeof(float2);
   const uint32_t tw = 16u * (uint32_t)k;
   geo.n_tiles = (a.d_hi - a.d_lo + 1 + tw - 1) / tw;
-  switch (k) {
-    case 4: return launch_perwin16<4>(groups, a, geo, smem, st);
-    case 2: return launch_perwin16<2>(groups, a, geo, smem, st);
-    default: return launch_perwin16<1>(groups, a, geo, smem, st);
-  }
+  const uint64_t want = (geo.n_tiles + groups - 1) / groups;
+  return dispatch(k, std::integer_sequence<int, 1, 2, 4>{}, [&](auto K) {
+    return launch_persistent("iqbb_fold_f32_perwin_kernel", iqbb_fold_f32_perwin16_kernel<K>, want > 0 ? want : 1, groups * kPwGroup, smem, st, a, geo);
+  }, [&] { return set_error(SDRG_ERR_RUNTIME, "IQBaseBand<float>: no per-window kernel for %d windows per half warp", k); });
 }
 
 }  // namespace sdrg

@@ -17,7 +17,7 @@
 // Kernel 2 (iqbb_finalize_*): one thread per completed window: division / narrowing, optional
 //   fused FM/AM/USB demodulation, carries the open window into the next call.
 #include "iqbb_int_common.cuh"
-#include <atomic>
+#include "launch.cuh"
 #include "demod_math.cuh"
 
 namespace sdrg {
@@ -323,29 +323,13 @@ int launch_fixed(const IqbbAccumArgs &a, const IqbbTaps &taps, unsigned n_tiles,
   constexpr int NV = (LP + 7 + 3) / 4;
   constexpr int xs_pitch = (kTile + 4 * NV + 8 + 3) & ~3;
   const size_t smem = sizeof(int2) * 128 + sizeof(int2) * kR * kZRow + sizeof(uint32_t) * 2 * xs_pitch;
-  static std::atomic<int> resident_dev[kMaxDevices];      // per instantiation and device: CTAs that fit at once
-  const int dev = current_device();
-  if (!resident_dev[dev]) {
-    int sms = 0, per_sm = 0;
-    SDRG_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    SDRG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, iqbb_accum_int_fixed_kernel<LP, VAR>, kT, smem));
-    resident_dev[dev] = sms * (per_sm > 0 ? per_sm : 1);
-  }
-  const unsigned grid = n_tiles < (unsigned)resident_dev[dev] ? n_tiles : (unsigned)resident_dev[dev];
-  iqbb_accum_int_fixed_kernel<LP, VAR><<<grid, kT, smem, st>>>(a, taps);
-  SDRG_CHECK_LAUNCH("iqbb_accum_int_fixed_kernel");
-  return SDRG_OK;
+  return launch_persistent("iqbb_accum_int_fixed_kernel", iqbb_accum_int_fixed_kernel<LP, VAR>, n_tiles, kT, smem, st, a, taps);
 }
 
 template <int VAR>
 int dispatch_fixed(int lp, const IqbbAccumArgs &a, const IqbbTaps &taps, unsigned grid, cudaStream_t st) {
-  switch (lp) {
-#define SDRG_CASE(N) case N: return launch_fixed<N, VAR>(a, taps, grid, st);
-    SDRG_CASE(2) SDRG_CASE(4) SDRG_CASE(6) SDRG_CASE(8) SDRG_CASE(10) SDRG_CASE(12) SDRG_CASE(14) SDRG_CASE(16)
-    SDRG_CASE(18) SDRG_CASE(20) SDRG_CASE(22) SDRG_CASE(24) SDRG_CASE(26) SDRG_CASE(28) SDRG_CASE(30) SDRG_CASE(32)
-#undef SDRG_CASE
-  }
-  return set_error(SDRG_ERR_RUNTIME, "no fixed-tap kernel for %d taps", lp);
+  return dispatch(lp, int_range<2, 32, 2>{}, [&](auto LP) { return launch_fixed<LP, VAR>(a, taps, grid, st); },
+                  [&] { return set_error(SDRG_ERR_RUNTIME, "no fixed-tap kernel for %d taps", lp); });
 }
 
 // ---- float kernel (direct form; the folded fast path lives in iqbb_fold_kernels.cu) ---------------
@@ -486,39 +470,17 @@ int launch_iqbb_accum(int scalar, const IqbbAccumArgs &a, cudaStream_t st) {
     if (scalar == SDRG_T_S8) return dispatch_fixed<1>(lp, a, taps, grid, st);
     return a.in_fmt == 4 ? dispatch_fixed<2>(lp, a, taps, grid, st) : dispatch_fixed<0>(lp, a, taps, grid, st);
   }
-  if (scalar == SDRG_T_F32) {
-    const size_t smem = accum_smem_f32(a.taps_len, a.hist_len);
-    if (smem > 48 * 1024)
-      SDRG_CUDA(cudaFuncSetAttribute(iqbb_accum_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    iqbb_accum_f32_kernel<<<grid, kT, smem, st>>>(a);
-    SDRG_CHECK_LAUNCH("iqbb_accum_f32_kernel");
-  } else {
-    const size_t smem = accum_smem_int(a.taps_len, a.hist_len);
-    if (scalar == SDRG_T_S8) {
-      if (smem > 48 * 1024)
-        SDRG_CUDA(cudaFuncSetAttribute(iqbb_accum_int_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      iqbb_accum_int_kernel<true><<<grid, kT, smem, st>>>(a);
-    } else {
-      if (smem > 48 * 1024)
-        SDRG_CUDA(cudaFuncSetAttribute(iqbb_accum_int_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      iqbb_accum_int_kernel<false><<<grid, kT, smem, st>>>(a);
-    }
-    SDRG_CHECK_LAUNCH("iqbb_accum_int_kernel");
-  }
-  return SDRG_OK;
+  if (scalar == SDRG_T_F32) return launch("iqbb_accum_f32_kernel", iqbb_accum_f32_kernel, grid, kT, accum_smem_f32(a.taps_len, a.hist_len), st, a);
+  return launch("iqbb_accum_int_kernel", scalar == SDRG_T_S8 ? iqbb_accum_int_kernel<true> : iqbb_accum_int_kernel<false>, grid, kT,
+                accum_smem_int(a.taps_len, a.hist_len), st, a);
 }
 
 int launch_iqbb_finalize(int scalar, const IqbbFinalizeArgs &a, cudaStream_t st) {
   const unsigned grid = (unsigned)((a.n_out + 255) / 256);
   const unsigned g = grid ? grid : 1;     // the carry must be moved even when nothing completed
-  switch (scalar) {
-    case SDRG_T_S16: iqbb_finalize_kernel<SDRG_T_S16><<<g, 256, 0, st>>>(a); break;
-    case SDRG_T_S8: iqbb_finalize_kernel<SDRG_T_S8><<<g, 256, 0, st>>>(a); break;
-    case SDRG_T_F32: iqbb_finalize_kernel<SDRG_T_F32><<<g, 256, 0, st>>>(a); break;
-    default: return set_error(SDRG_ERR_ARG, "finalize: unsupported scalar %d", scalar);
-  }
-  SDRG_CHECK_LAUNCH("iqbb_finalize_kernel");
-  return SDRG_OK;
+  return dispatch(scalar, std::integer_sequence<int, SDRG_T_S16, SDRG_T_S8, SDRG_T_F32>{},
+                  [&](auto S) { return launch("iqbb_finalize_kernel", iqbb_finalize_kernel<S>, g, 256, 0, st, a); },
+                  [&] { return set_error(SDRG_ERR_ARG, "finalize: unsupported scalar %d", scalar); });
 }
 
 }  // namespace sdrg

@@ -21,8 +21,7 @@
 // 0 Hz, the sdr_rec configuration -- two multiplies per tap), 4 real taps SYMMETRIC about the middle of an even count
 // (pairs of samples are added first: one multiply per component and tap pair; (x_a + x_b) k = x_a k + x_b k in Z/2^32).
 #include "iqbb_int_common.cuh"
-
-#include <atomic>
+#include "launch.cuh"
 
 namespace sdrg {
 namespace {
@@ -267,31 +266,14 @@ int launch_warp(IqbbAccumArgs a, const IqbbTaps &taps, cudaStream_t st) {
   constexpr int NV = (LP + 7 + 3) / 4;
   constexpr int pitch = ((kWT - kR + 4 * NV) + 7) & ~7;
   const size_t smem = sizeof(int2) * 128 + sizeof(int2) * (kT / 32) * 32 + sizeof(uint32_t) * (kT / 32) * 2 * pitch;
-  static std::atomic<int> resident_dev[kMaxDevices];
-  const int dev = current_device();
-  if (!resident_dev[dev]) {
-    int sms = 0, per_sm = 0;
-    SDRG_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    SDRG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, iqbb_accum_int_warp_kernel<LP, VAR, CONV>, kT, smem));
-    resident_dev[dev] = sms * (per_sm > 0 ? per_sm : 1);
-  }
   magic_div(a.ss, &a.div_m, &a.div_s);
   const unsigned n_tiles = (a.n + kWT - 1) / kWT, want = (n_tiles + kT / 32 - 1) / (kT / 32);
-  const unsigned grid = want < (unsigned)resident_dev[dev] ? want : (unsigned)resident_dev[dev];
-  iqbb_accum_int_warp_kernel<LP, VAR, CONV><<<grid, kT, smem, st>>>(a, taps);
-  SDRG_CHECK_LAUNCH("iqbb_accum_int_warp_kernel");
-  return SDRG_OK;
+  return launch_persistent("iqbb_accum_int_warp_kernel", iqbb_accum_int_warp_kernel<LP, VAR, CONV>, want, kT, smem, st, a, taps);
 }
 
 template <int VAR, bool CONV>
 int dispatch_warp(int lp, const IqbbAccumArgs &a, const IqbbTaps &taps, cudaStream_t st) {
-  switch (lp) {
-#define SDRG_CASE(N) case N: return launch_warp<N, VAR, CONV>(a, taps, st);
-    SDRG_CASE(2) SDRG_CASE(4) SDRG_CASE(6) SDRG_CASE(8) SDRG_CASE(10) SDRG_CASE(12) SDRG_CASE(14) SDRG_CASE(16)
-    SDRG_CASE(18) SDRG_CASE(20) SDRG_CASE(22) SDRG_CASE(24) SDRG_CASE(26) SDRG_CASE(28) SDRG_CASE(30) SDRG_CASE(32)
-#undef SDRG_CASE
-  }
-  return -1;
+  return dispatch(lp, int_range<2, 32, 2>{}, [&](auto LP) { return launch_warp<LP, VAR, CONV>(a, taps, st); }, [] { return -1; });
 }
 
 }  // namespace
