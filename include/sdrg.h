@@ -52,9 +52,9 @@ typedef struct {
 
 /* ---- runtime ---------------------------------------------------------------------------------- */
 int         sdrg_abi_version(void);
-/* 1 if the library was built with -DSDRG_EXPERIMENTS (environment-variable tuning switches, bandwidth probes and
- * the TMA staging variant of the float kernel compiled in); 0 for the shipped build, in which no environment
- * variable can change what is computed.  Returns the flag itself, not a status. */
+/* Always 0: the library is built one way only, and no environment variable can change what it computes or which
+ * kernel it launches.  Kept so that existing callers of this check keep working.  Returns the flag itself, not a
+ * status. */
 int         sdrg_build_has_experiments(void);
 const char *sdrg_last_error(void);
 int         sdrg_device_count(int *count);
@@ -126,16 +126,15 @@ int sdrg_iqbb_set_input_type(sdrg_iqbb *h, int type);
 
 /* SDRG_T_F32 only: which accumulate kernel config() selects.  0 = auto (folded when
  * sub_sample >= max(2, order-1), else direct), 1 = direct (sample-by-sample FIR, FMA-bound),
- * 2 = folded (one weight per input sample, HBM-bound; SDRG_ERR_CONFIG at config() if not eligible),
- * 3 = folded with TMA bulk-copy staging through shared memory (same results; only in builds with
- *     SDRG_EXPERIMENTS, otherwise SDRG_ERR_CONFIG).
+ * 2 = folded (one weight per input sample, HBM-bound; SDRG_ERR_CONFIG at config() if not eligible).
+ * 3 (formerly folded with TMA bulk-copy staging) is refused with SDRG_ERR_CONFIG.
  * Must be called before config(). */
 int sdrg_iqbb_set_float_path(sdrg_iqbb *h, int mode);
 
 /* Diagnostics (no reference counterpart): which accumulate kernel the node's last process() call launched.
  * 0 = none yet / integer node, 1 = direct FIR, 2 = folded (batched, any window length), 3 = folded, window-pipelined
  * (sub_sample <= 512), 4 = folded, staged short windows, 5 = folded, one thread group per window
- * (iqbb_fold_perwin.cu), 6 = folded, TMA staging (SDRG_EXPERIMENTS builds). */
+ * (iqbb_fold_perwin.cu).  6 (formerly folded, TMA staging) is no longer returned. */
 int sdrg_iqbb_last_float_kernel(const sdrg_iqbb *h, int *which);
 
 /* What config() derived; kernel/lut are written only when non-NULL (order / 128 int32 pairs, resp.

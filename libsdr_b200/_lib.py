@@ -209,10 +209,6 @@ def profile_read(kind):
     return ms.value, n.value
 
 
-def has_experiments():
-    return bool(load().sdrg_build_has_experiments())
-
-
 def kernel_launch_count():
     n = C.c_uint64(0)
     call("sdrg_kernel_launch_count", C.byref(n))

@@ -12,11 +12,10 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libsdrg.so")
-EXPERIMENTS = os.environ.get("SDRG_EXPERIMENTS", "0") not in ("", "0")     # probes / ablations / tuning switches: not shipped
-SOURCES = ["api.cu", "launch.cu", "design.cc", "iqbb_kernels.cu", "iqbb_warp_kernels.cu", "iqbb_fold_kernels.cu", "iqbb_fold_perwin.cu"] + (["iqbb_fold_experimental.cu"] if EXPERIMENTS else []) + ["demod_kernels.cu",
+SOURCES = ["api.cu", "launch.cu", "design.cc", "iqbb_kernels.cu", "iqbb_warp_kernels.cu", "iqbb_fold_kernels.cu", "iqbb_fold_perwin.cu", "demod_kernels.cu",
            "fft_kernels.cu", "fft8k_kernels.cu", "conv8k_kernels.cu", "fft_general.cu", "fft_api.cu", "bank_kernels.cu", "bank_api.cu", "multi_gpu.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
-              "-Xcompiler", "-fPIC,-O3,-fwrapv,-fno-fast-math", "-shared", "-cudart", "static"] + (["-DSDRG_EXPERIMENTS"] if EXPERIMENTS else [])
+              "-Xcompiler", "-fPIC,-O3,-fwrapv,-fno-fast-math", "-shared", "-cudart", "static"]
 
 
 def sources():
@@ -41,7 +40,7 @@ def needs_build():
     if not os.path.exists(OUT):
         return True
     if not os.path.exists(_stamp()) or open(_stamp()).read() != " ".join(_compile_flags()):
-        return True                          # built with other flags (e.g. SDRG_EXPERIMENTS)
+        return True                          # built with other flags (e.g. SDRG_NVCC_EXTRA)
     t = os.path.getmtime(OUT)
     return any(os.path.getmtime(d) > t for d in sources() + _headers())
 

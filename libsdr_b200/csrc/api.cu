@@ -402,7 +402,7 @@ int run_call(sdrg_iqbb *h, const void *d_in, uint32_t n, void *d_bb, void *d_aud
     fa.v_rows = h->v_rows; fa.v_pitch = h->v_pitch;
     fa.n = n; fa.taps_len = (uint32_t)h->d.order; fa.ss = a.ss; fa.r0 = a.r0; fa.first = a.first;
     fa.phase0 = a.nco ? a.phase0 : 0u; fa.inc = a.nco ? a.inc : 0u;
-    fa.zero_next = a.zero_next; fa.variant = h->float_path == 3 ? 2u : 0u;
+    fa.zero_next = a.zero_next;
     fa.work = h->d_work; f.work_reset = h->d_work;
     ProfScope ps(SDRG_KERNEL_IQBB_ACCUM, st);
     rc = launch_iqbb_fold(fa, st, &h->last_float_kernel);
@@ -449,13 +449,7 @@ int config_common(const char *who, int expect_type, const sdrg_config *src, bool
 extern "C" {
 
 int sdrg_abi_version(void) { return SDRG_ABI_VERSION; }
-int sdrg_build_has_experiments(void) {
-#ifdef SDRG_EXPERIMENTS
-  return 1;
-#else
-  return 0;
-#endif
-}
+int sdrg_build_has_experiments(void) { return 0; }
 const char *sdrg_last_error(void) { return g_err; }
 
 int sdrg_device_count(int *count) {
@@ -843,10 +837,8 @@ int sdrg_iqbb_set_input_type(sdrg_iqbb *h, int type) {
 
 int sdrg_iqbb_set_float_path(sdrg_iqbb *h, int mode) {
   if (!h) return set_error(SDRG_ERR_ARG, "null handle");
-  if (mode < 0 || mode > 3) return set_error(SDRG_ERR_ARG, "IQBaseBand: float path must be 0 (auto), 1 (direct), 2 (folded) or 3 (folded, TMA staging)");
-#ifndef SDRG_EXPERIMENTS
-  if (mode == 3) return set_error(SDRG_ERR_CONFIG, "IQBaseBand: the TMA staging variant exists only in builds made with SDRG_EXPERIMENTS=1");
-#endif
+  if (mode == 3) return set_error(SDRG_ERR_CONFIG, "IQBaseBand: there is no float path 3 (the TMA staging variant was removed)");
+  if (mode < 0 || mode > 2) return set_error(SDRG_ERR_ARG, "IQBaseBand: float path must be 0 (auto), 1 (direct) or 2 (folded)");
   if (h->configured) return set_error(SDRG_ERR_RUNTIME, "IQBaseBand: select the float path before config()");
   h->float_path = mode;
   return SDRG_OK;

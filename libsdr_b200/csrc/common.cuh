@@ -31,16 +31,6 @@ void count_launch(unsigned n = 1);                      // kernel launch counter
     ::sdrg::count_launch();                                                                     \
   } while (0)
 
-// Tuning / diagnostic switches read from the environment exist only in builds made with -DSDRG_EXPERIMENTS
-// (python -m libsdr_b200.build with SDRG_EXPERIMENTS=1).  The shipped library always takes the default:
-// no environment variable can change what it computes or which kernel it launches.
-#ifdef SDRG_EXPERIMENTS
-#include <cstdlib>
-static inline int env_int(const char *name, int dflt) { const char *e = getenv(name); return e ? atoi(e) : dflt; }
-#else
-static inline int env_int(const char *, int dflt) { return dflt; }
-#endif
-
 // ---- scalar helpers ---------------------------------------------------------------------------
 static inline size_t scalar_bytes(int scalar) {
   switch (scalar) {

@@ -21,7 +21,6 @@
 #include "fft_kernels.cuh"
 #include "fft_device.cuh"
 #include "launch.cuh"
-#include <cstdlib>
 
 namespace sdrg {
 namespace {
@@ -169,20 +168,6 @@ __device__ __forceinline__ void stage_inplace(float2 *__restrict__ buf, const in
   if (!DST_G) __syncthreads();
 }
 
-// n = EPT * blockDim.x points: EPT/8 radix-8, EPT/4 radix-4 or EPT/2 radix-2 butterflies per thread
-template <bool INV, int EPT>
-__device__ void fft_smem_inplace(float2 *buf, const int n, const int log2n, const float2 *tw, const float2 *mul) {
-  int Ns = 1, left = log2n;
-  bool first = true;
-  while (left > 0) {
-    const float2 *m = first ? mul : nullptr;
-    if (left >= 3 && left != 4) { stage_inplace<8, INV, EPT / 8>(buf, n, Ns, tw, m, threadIdx.x, blockDim.x); Ns *= 8; left -= 3; }
-    else if (left >= 2) { stage_inplace<4, INV, EPT / 4>(buf, n, Ns, tw, m, threadIdx.x, blockDim.x); Ns *= 4; left -= 2; }
-    else { stage_inplace<2, INV, EPT / 2>(buf, n, Ns, tw, m, threadIdx.x, blockDim.x); Ns *= 2; left -= 1; }
-    first = false;
-  }
-}
-
 // Stages for the middle `bits` bits of a transform whose first (forward) or last (inverse) radix-2
 // stage is fused into the global load / store: radix 16 while possible, then 8 / 4 / 2.
 template <bool INV>
@@ -250,30 +235,6 @@ __global__ void __launch_bounds__(512, 2) filter_ola1_r16_kernel(const FilterArg
     const float2 v = csubf(s0[pidx(j)], cmulf(s0[pidx(N + j)], w));
     o[j] = make_float2(v.x * sc, v.y * sc);
   }
-}
-
-// Single-filter overlap-save with one shared buffer: 16 elements per thread, 512 threads and 72 KB
-// at block 4096 -> two (register-limited) resident CTAs per SM whose barrier phases overlap.
-__global__ void __launch_bounds__(512, 2) filter_ola1_kernel(const FilterArgs a) {
-  extern __shared__ __align__(16) unsigned char fft_smem_raw[];
-  const int N = a.block, n = 2 * N;
-  float2 *s0 = (float2 *)fft_smem_raw;
-  const int b = blockIdx.x;
-  const float2 *x = (const float2 *)a.x;
-  const float2 *prev = b == 0 ? (const float2 *)a.hist_in : x + (size_t)(b - 1) * N;
-  const float2 *cur = x + (size_t)b * N;
-  for (int i = threadIdx.x; i < N; i += blockDim.x) { s0[pidx(i)] = prev[i]; s0[pidx(N + i)] = cur[i]; }
-  if (b == (int)gridDim.x - 1) {
-    float2 *ho = (float2 *)a.hist_out;
-    for (int i = threadIdx.x; i < N; i += blockDim.x) ho[i] = cur[i];
-  }
-  __syncthreads();
-  const float2 *tw = (const float2 *)a.tw;
-  fft_smem_inplace<false, 16>(s0, n, a.log2n, tw, nullptr);
-  fft_smem_inplace<true, 16>(s0, n, a.log2n, tw, (const float2 *)a.kern);
-  const float sc = 1.0f / (float)n;
-  float2 *o = (float2 *)a.out + (size_t)b * N;
-  for (int i = threadIdx.x; i < N; i += blockDim.x) { const float2 v = s0[pidx(N + i)]; o[i] = make_float2(v.x * sc, v.y * sc); }
 }
 
 // ---- batched plain FFT (FFTPlan<float>::operator()) ---------------------------------------------
@@ -362,8 +323,7 @@ __global__ void __launch_bounds__(1024) filter_ola_kernel(const FilterArgs a) {
 
 int launch_fft_batch(const void *in, void *out, int n, int log2n, int inverse, size_t batch, const void *tw, cudaStream_t st) {
   if (batch == 0) return SDRG_OK;
-  static const int r16 = env_int("SDRG_FFT_R16", 1);
-  if (r16 && n >= 256 && batch <= 0x7fffffffull) {
+  if (n >= 256 && batch <= 0x7fffffffull) {
     const int tpf = n / 16, fpc = tpf >= 256 ? 1 : 256 / tpf;
     const size_t smem = (size_t)fpc * padded_len(n) * sizeof(float2);
     return launch("fft_batch_r16_kernel", inverse ? fft_batch_r16_kernel<true> : fft_batch_r16_kernel<false>, (unsigned)((batch + fpc - 1) / fpc),
@@ -378,10 +338,8 @@ int launch_filter_ola(const FilterArgs &a, size_t n_blocks, cudaStream_t st) {
   if (n_blocks == 0) return SDRG_OK;
   const int n = 2 * a.block;
   if (n == 8192 && a.n_filters >= 1 && a.kperm && a.tab8k) return launch_conv8k(a, n_blocks, st);
-  static const int r16 = env_int("SDRG_FFT_R16", 1);
-  if (n >= 512 && (a.n_filters == 1 || (r16 && a.spec))) {   // in-place stages on a single buffer (n == 16 * threads)
+  if (n >= 512 && (a.n_filters == 1 || a.spec)) {   // in-place stages on a single buffer (n == 16 * threads)
     const size_t smem1 = (size_t)padded_len(n) * sizeof(float2);
-    if (!r16) return launch("filter_ola1_kernel", filter_ola1_kernel, (unsigned)n_blocks, n / 16, smem1, st, a);
     if (a.n_filters == 1) return launch("filter_ola1_r16_kernel", filter_ola1_r16_kernel<0>, (unsigned)n_blocks, n / 16, smem1, st, a);
     // bank: one forward pass, then every (block, filter) pair on its own CTA
     const int rc = launch("filter_ola1_r16_kernel<fwd>", filter_ola1_r16_kernel<1>, (unsigned)n_blocks, n / 16, smem1, st, a);

@@ -1,9 +1,8 @@
-// iqbb_fold_common.cuh -- helpers shared by the folded float kernels (iqbb_fold_kernels.cu) and their
-// experimental / instrumentation variants (iqbb_fold_experimental.cu).  See iqbb_fold_kernels.cu for the method.
+// iqbb_fold_common.cuh -- helpers shared by the folded float kernels (iqbb_fold_kernels.cu, iqbb_fold_perwin.cu).
+// See iqbb_fold_kernels.cu for the method.
 #pragma once
 #include "iqbb_kernels.cuh"
 #include "launch.cuh"
-#include <cstdlib>
 
 namespace sdrg {
 namespace foldk {
@@ -16,12 +15,6 @@ __device__ __forceinline__ float2 ld_stream(const float2 *p) {
   float2 v;
   asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "l"(p));
   return v;
-}
-// bulk L2 prefetch of [p, p + bytes): one instruction, no registers held while the data is in flight
-__device__ __forceinline__ void prefetch_l2(const float2 *lo, const float2 *hi) {
-  const uintptr_t a = (reinterpret_cast<uintptr_t>(lo) + 15) & ~uintptr_t(15);
-  const uintptr_t b = reinterpret_cast<uintptr_t>(hi) & ~uintptr_t(15);
-  if (b > a) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a), "r"((uint32_t)(b - a)) : "memory");
 }
 __device__ __forceinline__ float2 cmul(float2 a, float2 b) {
   return make_float2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x);
@@ -93,16 +86,12 @@ __device__ __forceinline__ bool chunk_of(const IqbbFoldArgs &a, uint32_t id, int
 // (the per-window kernel computes whole windows itself and needs only one of the two from its neighbours);
 // STAGED = false reduces with shuffles and issues the RED.ADDs at once (no per-warp staging rows needed).
 template <bool STAGED = true>
-__device__ __forceinline__ void fold_chunk_general(const IqbbFoldArgs &a, const uint32_t id, const uint32_t total_warps,
+__device__ __forceinline__ void fold_chunk_general(const IqbbFoldArgs &a, const uint32_t id,
                                                    const float2 *__restrict__ x, const float2 *sA, const float2 *sH,
                                                    const int lane, const int L1, const int win_off,
                                                    const uint32_t inc32, const uint32_t inc256,
                                                    WarpStage &stage, float *acc_out, const uint32_t what = 3u) {
     Chunk c;
-    if (lane == 0 && a.pf_dist && id + a.pf_dist * total_warps < a.n_chunks) {   // a later chunk of this warp -> L2, one instruction
-      Chunk nx;
-      if (chunk_of(a, id + a.pf_dist * total_warps, win_off, L1, nx)) prefetch_l2(x + nx.c_lo, x + nx.c_lo + nx.len);
-    }
     if (!chunk_of(a, id, win_off, L1, c)) return;
     const int len = c.len;
     uint32_t ph = (a.phase0 + (uint32_t)(c.c_lo + lane) * a.inc) & 0x7fffu;         // this lane's phase in step 0
@@ -174,9 +163,5 @@ __device__ __forceinline__ void fold_chunk_general(const IqbbFoldArgs &a, const 
 // iqbb_fold_perwin.cu: whole windows per thread group (short windows); false when the call has no eligible window
 bool fold_perwin_eligible(IqbbFoldArgs &a);
 int launch_fold_perwin(const IqbbFoldArgs &a, cudaStream_t st);
-
-// iqbb_fold_experimental.cu
-int launch_fold_tma(IqbbFoldArgs a, cudaStream_t st);                 // opt-in TMA bulk-copy staging (float path 3)
-int launch_fold_probe(int mode, IqbbFoldArgs a, cudaStream_t st);     // SDRG_FOLD_PROBE bandwidth probes (instrumentation)
 
 }  // namespace sdrg

@@ -121,7 +121,7 @@ __global__ void __launch_bounds__(kFoldThreads, 4) iqbb_fold_f32_kernel(const Iq
       if (L1 > 0) stage.push(sent, id + 1, lane, acc_out);
       continue;
     }
-    fold_chunk_general(a, id, total_warps, x, sA, sH, lane, L1, win_off, inc32, inc256, stage, acc_out);
+    fold_chunk_general(a, id, x, sA, sH, lane, L1, win_off, inc32, inc256, stage, acc_out);
   }
   stage.drain(lane, acc_out);
 
@@ -134,7 +134,7 @@ __global__ void __launch_bounds__(kFoldThreads, 4) iqbb_fold_f32_kernel(const Iq
 // constant (S x 256 B) and a window costs no exposed memory round trip -- the two per window of the
 // batched schedule above were what kept it at ~92 % of HBM.  Edge chunks (window 0, the clipped
 // last window) go through fold_chunk_general.
-template <int S, int P = 0, int TS = 3>     // TS: ring steps that can hold tail samples (3: taps <= 65, 5: taps <= 129); P != 0: timing experiments only (bit 0 no tails, bit 1 no A lookup, bit 2 no H weighting)
+template <int S, int TS = 3>     // TS: ring steps that can hold tail samples (3: taps <= 65, 5: taps <= 129)
 __global__ void __launch_bounds__(kFoldThreads, S <= 8 ? 4 : (S <= 13 ? 3 : 2)) iqbb_fold_f32_win_kernel(const IqbbFoldArgs a) {
   extern __shared__ __align__(16) unsigned char dyn_smem[];
   __shared__ float2 sA[128];
@@ -146,7 +146,6 @@ __global__ void __launch_bounds__(kFoldThreads, S <= 8 ? 4 : (S <= 13 ? 3 : 2)) 
   sH[tid] = a.tab_u[(size_t)tid * a.taps_len];
   __syncthreads();
 
-  const uint32_t T = gridDim.x * kFoldWarps;
   const uint32_t wg = warp * gridDim.x + blockIdx.x;
   const float2 *__restrict__ x = (const float2 *)a.x;
   float *acc_out = (float *)a.acc_cur;
@@ -160,8 +159,8 @@ __global__ void __launch_bounds__(kFoldThreads, S <= 8 ? 4 : (S <= 13 ? 3 : 2)) 
   for (int k = 0; k < TS; ++k) { te[k] = (int)a.ss - 32 * (S - 1 - k) - lane; te_ok[k] = te[k] >= 1 && te[k] <= L1; }
 
   // Edge chunks (window 0, the clipped last window and the tails behind it) are dealt statically ...
-  if (wg == 0) fold_chunk_general(a, 0u, T, x, sA, sH, lane, L1, win_off, inc32, inc256, stage, acc_out);
-  else if (a.fast_hi + wg < a.n_chunks) fold_chunk_general(a, a.fast_hi + wg, T, x, sA, sH, lane, L1, win_off, inc32, inc256, stage, acc_out);
+  if (wg == 0) fold_chunk_general(a, 0u, x, sA, sH, lane, L1, win_off, inc32, inc256, stage, acc_out);
+  else if (a.fast_hi + wg < a.n_chunks) fold_chunk_general(a, a.fast_hi + wg, x, sA, sH, lane, L1, win_off, inc32, inc256, stage, acc_out);
   // ... the complete interior windows 1..fast_hi dynamically, kWorkChunk consecutive windows per grab of a
   // global counter: a CTA that becomes resident late (another kernel -- e.g. a collective -- holding part of
   // the SMs) or runs on a slower SM simply takes fewer windows, and ids still advance in address order.
@@ -201,7 +200,7 @@ __global__ void __launch_bounds__(kFoldThreads, S <= 8 ? 4 : (S <= 13 ? 3 : 2)) 
 #pragma unroll
       for (int k = 0; k < TS; ++k) {
         ut[k] = make_float2(0.f, 0.f);
-        if (!(P & 1) && k < S && te_ok[k]) ut[k] = (P & 8) ? Ab : __ldg(urow + te[k]);
+        if (k < S && te_ok[k]) ut[k] = __ldg(urow + te[k]);
       }
       float2 R[8];
 #pragma unroll
@@ -209,9 +208,8 @@ __global__ void __launch_bounds__(kFoldThreads, S <= 8 ? 4 : (S <= 13 ? 3 : 2)) 
       float2 ts = make_float2(0.f, 0.f);
 #pragma unroll
       for (int i = 0; i < S; ++i) {
-        if (P & 2) cfma(R[i & 7], Ab, ring[i]);
-        else cfma(R[i & 7], sA[((ph + i * inc32) & 0x7fffu) >> 8], ring[i]);
-        if (!(P & 1) && S - 1 - i < TS) cfma(ts, ut[S - 1 - i], ring[i]);    // zero weight outside the tail
+        cfma(R[i & 7], sA[((ph + i * inc32) & 0x7fffu) >> 8], ring[i]);
+        if (S - 1 - i < TS) cfma(ts, ut[S - 1 - i], ring[i]);    // zero weight outside the tail
         if (more) {
           if (i + 1 < S) ring[i] = ld_stream(xn + 32 * i);
           else if (last_ok) ring[i] = ld_stream(xn + 32 * i);    // lanes past the window keep their zero
@@ -221,16 +219,13 @@ __global__ void __launch_bounds__(kFoldThreads, S <= 8 ? 4 : (S <= 13 ? 3 : 2)) 
       float2 tot = make_float2(-sent.x, -sent.y);
       const uint32_t r0 = ph & 255u;
 #pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        if (P & 4) { tot.x += R[u].x; tot.y += R[u].y; }
-        else cfma(tot, sH[(r0 + u * inc32) & 255u], R[u]);
-      }
+      for (int u = 0; u < 8; ++u) cfma(tot, sH[(r0 + u * inc32) & 255u], R[u]);
       // the tails this window owes to the next one stay in registers while the warp walks consecutive windows
       // (15 of 16): one staged row per window instead of two
       tot.x += carry.x; tot.y += carry.y;
       stage.push(tot, id, lane, acc_out);
       carry = sent;
-      if ((!more || switched) && L1 > 0 && !(P & 1)) { stage.push(carry, id + 1, lane, acc_out); carry = make_float2(0.f, 0.f); }
+      if ((!more || switched) && L1 > 0) { stage.push(carry, id + 1, lane, acc_out); carry = make_float2(0.f, 0.f); }
       if (!more) break;
       if (switched) {
         end = min(nid + kWorkChunk, a.fast_hi + 1);
@@ -242,22 +237,17 @@ __global__ void __launch_bounds__(kFoldThreads, S <= 8 ? 4 : (S <= 13 ? 3 : 2)) 
   stage.drain(lane, acc_out);
 }
 
-template <int S, int P = 0, int TS = 3>
+template <int S, int TS = 3>
 static int launch_fold_win_s(const IqbbFoldArgs &a, cudaStream_t st) {
   const size_t smem = (size_t)kFoldWarps * kStageRows * kStagePitch * sizeof(float2);
   const uint64_t want = ((uint64_t)a.n_chunks + kFoldWarps - 1) / kFoldWarps;
-  return launch_persistent("iqbb_fold_f32_win_kernel", iqbb_fold_f32_win_kernel<S, P, TS>, want, kFoldThreads, smem, st, a);
+  return launch_persistent("iqbb_fold_f32_win_kernel", iqbb_fold_f32_win_kernel<S, TS>, want, kFoldThreads, smem, st, a);
 }
 
 static int launch_fold_win(const IqbbFoldArgs &a, cudaStream_t st) {
   const int s = (int)((a.ss + 31) / 32);
-#ifdef SDRG_EXPERIMENTS
-  static const int wp = env_int("SDRG_FOLD_WINP", 0);   // ablations of the S = 13 kernel: WRONG RESULTS, timing only
-  if (wp >= 1 && wp <= 8 && s == 13)
-    return dispatch(wp, int_range<1, 8>{}, [&](auto P) { return launch_fold_win_s<13, P>(a, st); }, [] { return SDRG_OK; });
-#endif
   if (a.taps_len > 65)        // 66..129 taps: the tail reaches back up to five ring steps (ss >= taps - 1 >= 65, so S >= 3)
-    return dispatch(s, int_range<3, 16>{}, [&](auto S) { return launch_fold_win_s<S, 0, 5>(a, st); }, [] {
+    return dispatch(s, int_range<3, 16>{}, [&](auto S) { return launch_fold_win_s<S, 5>(a, st); }, [] {
       return set_error(SDRG_ERR_RUNTIME, "IQBaseBand<float>: window-pipelined kernel needs 65 <= sub_sample <= 512 for more than 65 taps");
     });
   return dispatch(s, int_range<1, 16>{}, [&](auto S) { return launch_fold_win_s<S>(a, st); },
@@ -373,7 +363,11 @@ static int launch_fold_small(const IqbbFoldArgs &a, cudaStream_t st) {
 }  // namespace
 
 // Grids are sized to the machine: 148 SMs x 3 resident CTAs of 8 warps.
-static int launch_fold_ldg(IqbbFoldArgs a, cudaStream_t st, int *which) {
+int launch_iqbb_fold(const IqbbFoldArgs &a_in, cudaStream_t st, int *which_out) {
+  int which_local = 0;
+  int *which = which_out ? which_out : &which_local;
+  if (a_in.n == 0) return SDRG_OK;
+  IqbbFoldArgs a = a_in;
   // slots touched by this call: slot of the last sample + 1
   const uint64_t q_last = (uint64_t)a.r0 + (a.n - 1) - ((a.first && a.n > 1) ? 1 : 0);
   const uint64_t n_slots = q_last / a.ss + 1;
@@ -382,12 +376,8 @@ static int launch_fold_ldg(IqbbFoldArgs a, cudaStream_t st, int *which) {
   const uint64_t n_chunks = n_slots * a.cpw;
   if (n_chunks > 0xffffffffull) return set_error(SDRG_ERR_RUNTIME, "IQBaseBand<float>: too many windows in one call");
   a.n_chunks = (uint32_t)n_chunks;
-  a.chunks_per_warp = 0;
-  static const int pf = env_int("SDRG_FOLD_PF", 0);   // measured: no gain with round-robin chunks
-  a.pf_dist = (uint32_t)pf;
-  static const int fast_env = env_int("SDRG_FOLD_FAST", 1);
-  a.fast = (fast_env && a.cpw == 1 && a.taps_len <= 65 && a.ss + 1 >= a.taps_len) ? 1u : 0u;   // batched kernel: two tail steps
-  const bool win_ok = fast_env && a.cpw == 1 && a.taps_len <= 129 && a.ss + 1 >= a.taps_len && a.ss <= 512;   // window-pipelined: up to five
+  a.fast = (a.cpw == 1 && a.taps_len <= 65 && a.ss + 1 >= a.taps_len) ? 1u : 0u;   // batched kernel: two tail steps
+  const bool win_ok = a.cpw == 1 && a.taps_len <= 129 && a.ss + 1 >= a.taps_len && a.ss <= 512;   // window-pipelined: up to five
   a.fast_nb = a.ss / 256;
   a.fast_rs = (a.ss % 256 + 31) / 32;
   a.fast_pl = a.ss % 32 ? a.ss % 32 : 32;
@@ -396,42 +386,14 @@ static int launch_fold_ldg(IqbbFoldArgs a, cudaStream_t st, int *which) {
     const int64_t hi = ((int64_t)a.n + (int64_t)a.r0 - (int64_t)a.first) / (int64_t)a.ss - 1;
     a.fast_hi = hi >= 1 ? (uint32_t)hi : 0u;
   }
-  static const int win_env = env_int("SDRG_FOLD_WIN", 1);
-  static const int chunk_env = env_int("SDRG_FOLD_WORK_CHUNK", 16);
-  a.work_chunk = (uint32_t)(chunk_env > 0 ? chunk_env : 16);
-#ifdef SDRG_EXPERIMENTS
-  static const int probe = env_int("SDRG_FOLD_PROBE", 0);   // bandwidth probes: WRONG RESULTS, timing only
-#else
-  constexpr int probe = 0;
-#endif
-  static const int perwin_max = env_int("SDRG_FOLD_PERWIN_MAX", 256);   // longest window taken by the per-window kernel (iqbb_fold_perwin.cu)
-  if (!probe && a.cpw == 1 && (int)a.ss <= perwin_max && fold_perwin_eligible(a)) { *which = 5; return launch_fold_perwin(a, st); }
-  static const int small_env = env_int("SDRG_FOLD_SMALL", 55);   // largest ss taken by the short-window kernel (measured crossover with the window-pipelined one)
-  if (!probe && a.cpw == 1 && a.ss + 1 >= a.taps_len && (a.ss < 32 || (int)a.ss <= small_env)) { *which = 4; return launch_fold_small(a, st); }
-  if (!probe && win_env && win_ok && a.fast_hi >= 1) { *which = 3; return launch_fold_win(a, st); }
-#ifdef SDRG_EXPERIMENTS
-  if (probe >= 1 && probe <= 3) return launch_fold_probe(probe, a, st);
-#endif
+  a.work_chunk = 16;
+  if (a.cpw == 1 && fold_perwin_eligible(a)) { *which = 5; return launch_fold_perwin(a, st); }
+  // ss <= 55: the short-window kernel (measured crossover with the window-pipelined one)
+  if (a.cpw == 1 && a.ss + 1 >= a.taps_len && a.ss <= 55) { *which = 4; return launch_fold_small(a, st); }
+  if (win_ok && a.fast_hi >= 1) { *which = 3; return launch_fold_win(a, st); }
   *which = 2;
   const size_t smem = (size_t)kFoldWarps * kStageRows * kStagePitch * sizeof(float2);
   return launch_persistent("iqbb_fold_f32_kernel", iqbb_fold_f32_kernel, (n_chunks + kFoldWarps - 1) / kFoldWarps, kFoldThreads, smem, st, a);
 }
 
-int launch_iqbb_fold(const IqbbFoldArgs &a, cudaStream_t st, int *which_out) {
-  int which_local = 0;
-  int *which = which_out ? which_out : &which_local;
-  if (a.n == 0) return SDRG_OK;
-  // bulk async copies need 16-byte aligned global addresses; otherwise use the LDG variant
-  const bool aligned = (reinterpret_cast<uintptr_t>(a.x) & 15u) == 0;
-#ifdef SDRG_EXPERIMENTS
-  static const int env_variant = env_int("SDRG_FOLD_VARIANT", 0);
-  const int variant = a.variant ? (int)a.variant : env_variant;      // 2 = TMA staging (iqbb_fold_experimental.cu)
-  if (aligned && variant == 2 && a.ss >= 32) { *which = 6; return launch_fold_tma(a, st); }
-#else
-  (void)aligned;
-#endif
-  return launch_fold_ldg(a, st, which);
-}
-
 }  // namespace sdrg
-

@@ -123,7 +123,7 @@ __device__ __forceinline__ void perwin_edges(const IqbbFoldArgs &a, const Perwin
   for (uint32_t e = threadIdx.x >> 5; e < geo.n_edge; e += blockDim.x >> 5) {
     const uint32_t id = e < a.d_lo ? e : a.d_hi + (e - a.d_lo);
     const uint32_t what = e < a.d_lo ? (e + 1 < a.d_lo ? 3u : 1u) : (id == a.d_hi ? 2u : 3u);
-    fold_chunk_general<false>(a, id, 1u, (const float2 *)a.x, sA, sH, lane, L1, win_off, inc32, inc256, none, (float *)a.acc_cur, what);
+    fold_chunk_general<false>(a, id, (const float2 *)a.x, sA, sH, lane, L1, win_off, inc32, inc256, none, (float *)a.acc_cur, what);
   }
 }
 
@@ -332,7 +332,7 @@ __global__ void __launch_bounds__(1024, 1) iqbb_fold_f32_perwin16_kernel(const I
   }
 }
 
-static uint32_t pw1_max() { static const int v = env_int("SDRG_FOLD_PERWIN1_MAX", 22); return (uint32_t)v; }   // ss <= this: a thread per window; above: a half warp per window
+constexpr uint32_t kPw1MaxSs = 22;        // ss <= this: a thread per window; above: a half warp per window
 
 constexpr size_t kPwMaxSmem = 220 * 1024;
 
@@ -361,16 +361,13 @@ size_t tile_elems(const IqbbFoldArgs &a, int k, uint32_t *delta_out) {
 // 4 groups x 2 buffers beat 2 groups x 3 buffers by 1.3-1.7x), then the tile size.  Two buffers per group; the largest
 // K <= k_max that still lets four groups fit next to the table, else the K with the most groups.
 void shape16(const IqbbFoldArgs &a, size_t table, int *k_out, int *groups_out) {
-  static const int k_env = env_int("SDRG_FOLD_PERWIN_K", 0), groups_env = env_int("SDRG_FOLD_PERWIN_GROUPS", 0);
   int best_k = 1, best_g = 0;
   for (int k = k_max_of(a.ss); k >= 1; k >>= 1) {
-    if (k_env && k != k_env && (k_env == 1 || k_env == 2 || k_env == 4)) continue;
     int g = 4;
     while (g > 1 && (table + (size_t)g * 2 * tile_elems(a, k, nullptr)) * sizeof(float2) > kPwMaxSmem) g >>= 1;
     if (g > best_g) { best_g = g; best_k = k; }
     if (g == 4) break;
   }
-  if (groups_env >= 1 && groups_env < best_g) best_g = groups_env;
   *k_out = best_k; *groups_out = best_g > 0 ? best_g : 1;
 }
 
@@ -385,8 +382,8 @@ bool fold_perwin_eligible(IqbbFoldArgs &a) {
   const int64_t hi = ((int64_t)a.n - win_off) / ss - 1;        // (hi + 1) ss + win_off <= n
   if (hi < lo) return false;
   a.d_lo = (uint32_t)lo; a.d_hi = (uint32_t)hi;
-  if (((size_t)a.v_rows * a.v_pitch + 1 + 2 * tile_elems(a, a.ss <= pw1_max() ? 0 : 1, nullptr)) * sizeof(float2) > kPwMaxSmem) return false;
-  if (a.ss > pw1_max() && a.taps_len <= 129) {
+  if (((size_t)a.v_rows * a.v_pitch + 1 + 2 * tile_elems(a, a.ss <= kPw1MaxSs ? 0 : 1, nullptr)) * sizeof(float2) > kPwMaxSmem) return false;
+  if (a.ss > kPw1MaxSs && a.taps_len <= 129) {
     // a table that leaves room for fewer than four thread groups: the window-pipelined kernel is faster (measured, 2 groups:
     // ss 96 / 97 taps 2.7 vs 3.5 TB/s, 100 / 101 2.8 vs 3.3, 128 / 20 4.2 vs 4.3; 4 groups: 96 / 64 5.2 vs 3.5)
     int k = 1, groups = 1;
@@ -399,14 +396,14 @@ bool fold_perwin_eligible(IqbbFoldArgs &a) {
 int launch_fold_perwin(const IqbbFoldArgs &a_in, cudaStream_t st) {
   IqbbFoldArgs a = a_in;
   const uint64_t q_last = (uint64_t)a.r0 + (a.n - 1) - ((a.first && a.n > 1) ? 1 : 0);
-  a.part = 8192; a.cpw = 1; a.pf_dist = 0; a.fast = 0;
+  a.part = 8192; a.cpw = 1; a.fast = 0;
   a.n_chunks = (uint32_t)(q_last / a.ss + 1);
   PerwinGeom geo{};
   geo.n_edge = a.d_lo + (a.n_chunks > a.d_hi ? a.n_chunks - a.d_hi : 0u);
   geo.magic = (uint32_t)(((1ull << 32) + a.ss - 1) / a.ss);
   geo.stages = 2;
   const size_t table = ((size_t)a.v_rows * a.v_pitch + 1) & ~(size_t)1;
-  if (a.ss <= pw1_max()) {
+  if (a.ss <= kPw1MaxSs) {
     // small table, several CTAs per SM with two buffers each (measured: 3 CTAs x 2 buffers beat 2 CTAs x 3)
     geo.x_tile = (uint32_t)tile_elems(a, 0, &geo.delta);
     geo.pitch = a.ss + geo.delta;

@@ -56,10 +56,6 @@ struct IqbbFoldArgs {
   uint32_t      part;       // a window longer than this is cut into pieces (chunks)
   uint32_t      cpw;        // chunks per window
   uint32_t      n_chunks;   // windows touched by this call x cpw
-  uint32_t      chunks_per_warp;
-  uint32_t      pf_dist;    // L2 prefetch distance in chunks of the same warp (0 = off)
-  uint32_t      seg;        // TMA variant: samples per warp segment (multiple of 256)
-  uint32_t      variant;    // 0/1 LDG loads (default), 2 TMA bulk-copy staging (needs 16-byte aligned input)
   // specialised schedule of a complete interior window (cpw == 1, taps_len <= 65), see iqbb_fold_f32_kernel
   uint32_t      fast;       // 1 = use it
   uint32_t      fast_nb;    // full 256-sample batches per window (ss / 256)

@@ -105,7 +105,7 @@ class IQBaseBand:
         _lib.call("sdrg_iqbb_set_float_path", self._h, int(mode))
 
     def lastFloatKernel(self):
-        """Diagnostics: 1 direct FIR, 2 folded batched, 3 window-pipelined, 4 staged short windows, 5 per-window, 6 TMA."""
+        """Diagnostics: 1 direct FIR, 2 folded batched, 3 window-pipelined, 4 staged short windows, 5 per-window."""
         w = C.c_int(0)
         _lib.call("sdrg_iqbb_last_float_kernel", self._h, C.byref(w))
         return w.value

@@ -128,3 +128,23 @@ def test_shipped_library_has_no_result_changing_switches():
     with pytest.raises(_lib.ConfigError):
         _lib.call("sdrg_iqbb_set_float_path", h, 3)
     lib.sdrg_iqbb_destroy(h)
+
+
+def test_one_build_without_environment_switches():
+    """The library is built one way only: no C/C++/CUDA source reads the environment, and nothing in the package or
+    the header names a second (experiments) build."""
+    offenders = []
+    for base in ("libsdr_b200", "include"):
+        for dp, dirs, fs in os.walk(os.path.join(ROOT, base)):
+            dirs[:] = [d for d in dirs if d != "__pycache__"]
+            for f in fs:
+                path = os.path.join(dp, f)
+                rel = os.path.relpath(path, ROOT)
+                text = open(path, encoding="utf-8", errors="replace").read()
+                native = f.endswith((".cu", ".cuh", ".cc", ".cpp", ".c", ".h", ".hh")) and \
+                    (base == "include" or rel.startswith(os.path.join("libsdr_b200", "csrc")))
+                if native and "getenv" in text:
+                    offenders.append((rel, "getenv"))
+                if "SDRG_EXPERIMENTS" in text:
+                    offenders.append((rel, "SDRG_EXPERIMENTS"))
+    assert not offenders, offenders

@@ -308,10 +308,8 @@ def _float_case(cfg, x, bs, demod=DEMOD_FM, path=0):
 PATHS = [(1, "direct"), (2, "folded")]
 
 
-@pytest.mark.parametrize("path", [1, 2, 3], ids=["direct", "folded", "folded-tma"])
+@pytest.mark.parametrize("path", [1, 2], ids=["direct", "folded"])
 def test_c2_float_chain(path):
-    if path == 3 and not _lib.has_experiments():
-        pytest.skip("the TMA staging variant is compiled only with SDRG_EXPERIMENTS=1")
     cfg = dict(synth.C2)
     x = synth.c2_input(2 << 20)
     e = _float_case(cfg, x, 1 << 20, DEMOD_FM, path)
@@ -335,7 +333,7 @@ def test_float_small_configs(demod, path):
 @pytest.mark.parametrize("ss,order", [(32, 33), (33, 2), (63, 64), (64, 64), (100, 2), (416, 1), (417, 64), (512, 65), (513, 65), (600, 40),
                                       (127, 128), (130, 129), (200, 129), (300, 66), (416, 128), (512, 100), (512, 129), (513, 129), (416, 130),
                                       (768, 64), (1000, 64), (2083, 15), (5000, 64), (8191, 64), (8192, 64), (8193, 64), (300000, 128)])
-@pytest.mark.parametrize("path", [2, 3], ids=["folded", "folded-tma"])
+@pytest.mark.parametrize("path", [2], ids=["folded"])
 def test_float_folded_geometry(ss, order, path):
     """Folded kernel across window/segment geometries (window << segment, window >> segment,
     ss == order-1, order 1), ragged multi-call streams."""
@@ -344,8 +342,6 @@ def test_float_folded_geometry(ss, order, path):
     cfg = dict(scalar="f32", Fs=20e6, Fc=1.25e6, Ff=1.2e6, width=200e3, order=order, sub_sample=ss, oFs=0.0)
     n = 700000
     x = synth.iq_f32(n, 20e6, [(0.5, 1.25e6, 0.3), (0.3, -4e6, 1.0)], 0.02, 11)
-    if path == 3 and not _lib.has_experiments():
-        pytest.skip("the TMA staging variant is compiled only with SDRG_EXPERIMENTS=1")
     g, o = gpu_bb(cfg, bs=n, float_path=path), orc_bb(cfg, bs=n)
     cuts = [0, 1, 31, 32, 33, 2047, 2048, 2049, 100000, 100001, 400000, n]
     ys, os_ = [], []
