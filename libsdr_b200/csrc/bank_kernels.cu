@@ -2,7 +2,8 @@
 // (BASELINE configs 4/5: 256..2048 channels with independent NCO offsets on a 100 MS/s stream).
 //
 // Every channel is an independent IQBaseBand (src/baseband.hh:198-236) fed the same buffers; the
-// arithmetic per channel is exactly that of iqbb_accum_int_kernel (bit-exact).  What changes is
+// arithmetic per channel is iqbb_int_common.cuh's (load_sample, fir_smem / fir_fixed, fir_result,
+// nco_mix, bit-exact), as in the single-channel kernels.  What changes is
 // the data movement: a CTA stages one 2048-sample input tile (+ halo) in shared memory ONCE and
 // loops over a group of channels (taps of the whole group preloaded in shared memory), so the
 // input is read from HBM once per channel group instead of once per channel; the work is purely
@@ -11,18 +12,15 @@
 // warp's 256 touch at most two windows, so window sums are formed in registers and reduced with
 // REDUX.SUM -- no shared-memory staging and no CTA barrier inside the channel loop.
 // IQBaseBand<float> channels take the folded kernel further below (bank_fold_f32_kernel).
-#include "iqbb_kernels.cuh"
+#include "iqbb_int_common.cuh"
 #include "iqbb_finalize.cuh"
 #include "iqbb_fold_common.cuh"
 
 namespace sdrg {
 namespace {
 
-constexpr int kT = kIqbbThreads, kR = kIqbbPerThread, kTile = kIqbbTile;
+constexpr int kT = kIqbbThreads, kTile = kIqbbTile;
 constexpr unsigned kFull = 0xffffffffu;
-
-__device__ __forceinline__ int pad32(int i) { return i + (i >> 5); }
-__device__ __forceinline__ void unpack16(uint32_t v, int &re, int &im) { re = (int)(short)(v & 0xffffu); im = ((int)v) >> 16; }
 
 template <bool IS_S8>
 __global__ void __launch_bounds__(kT) bank_accum_kernel(const BankAccumArgs a) {
@@ -36,106 +34,52 @@ __global__ void __launch_bounds__(kT) bank_accum_kernel(const BankAccumArgs a) {
   int2 *lut = (int2 *)(tp + (size_t)a.group * Lp);               // 128
   uint32_t *xs = (uint32_t *)(lut + 128);                        // pad32(n_xs)+1
 
-  // prologue shared with the single-channel kernel: zero next accumulators, roll the history
-  {
-    int2 *nxt = (int2 *)a.acc_next;
-    const size_t total = (size_t)a.zero_next * a.channels;       // per channel: first zero_next slots
-    const size_t stride = (size_t)gridDim.x * gridDim.y * blockDim.x;
-    for (size_t k = ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * blockDim.x + tid; k < total; k += stride)
-      nxt[(k / a.zero_next) * a.acc_stride + (k % a.zero_next)] = make_int2(0, 0);
-    if (blockIdx.x == 0 && blockIdx.y == 0) {
-      const int64_t n = a.n;
-      for (int64_t k = tid; k < H; k += blockDim.x) {
-        const int64_t i = n - H + k;
-        if (IS_S8) ((char2 *)a.hist_out)[k] = (i >= 0) ? ((const char2 *)a.x)[i] : ((const char2 *)a.hist_in)[H + i];
-        else ((uint32_t *)a.hist_out)[k] = (i >= 0) ? ((const uint32_t *)a.x)[i] : ((const uint32_t *)a.hist_in)[H + i];
-      }
-    }
-  }
+  if (IS_S8) bank_prologue<char2>(a, tid); else bank_prologue<uint32_t>(a, tid);
 
   const int64_t tile_base = (int64_t)blockIdx.x * kTile;
   for (int k = tid; k < nch * Lp; k += kT) tp[k] = ((const int4 *)a.taps)[(size_t)c0 * Lp + k];
   if (tid < 128) lut[tid] = ((const int2 *)a.lut)[tid];
-  for (int k = tid; k < n_xs; k += kT) {
-    const int64_t i = tile_base - H + k;
-    uint32_t v = 0;
-    if (IS_S8) {
-      char2 s = make_char2(0, 0);
-      if (i < 0) s = ((const char2 *)a.hist_in)[H + i];
-      else if (i < (int64_t)a.n) s = ((const char2 *)a.x)[i];
-      v = ((uint32_t)(uint16_t)(int16_t)s.x) | (((uint32_t)(uint16_t)(int16_t)s.y) << 16);
-    } else {
-      if (i < 0) v = ((const uint32_t *)a.hist_in)[H + i];
-      else if (i < (int64_t)a.n) v = ((const uint32_t *)a.x)[i];
-    }
-    xs[pad32(k)] = v;
-  }
+  for (int k = tid; k < n_xs; k += kT) xs[pad32(k)] = load_sample<IS_S8>(a.x, a.hist_in, tile_base - H + k, H, a.n, 0u);
   __syncthreads();
 
   // window geometry of this thread's 8 outputs (identical for every channel)
   const int ob = tid * kR;
   const uint32_t i0 = (uint32_t)tile_base + (uint32_t)ob;        // call-relative index of output 0
   const uint32_t tile_hi = (uint32_t)min((int64_t)a.n, tile_base + kTile);
-  const uint64_t q0 = (uint64_t)a.r0 + i0 - ((a.first && i0 > 0) ? 1u : 0u);
-  const uint32_t slot_a = (uint32_t)(q0 / a.ss);
-  // first call-relative index that belongs to slot_a + 1
-  const int64_t bnd = (int64_t)((uint64_t)(slot_a + 1) * a.ss) - (int64_t)a.r0 + (int64_t)a.first;
-  const uint32_t w_i0 = (uint32_t)tile_base + (uint32_t)((tid & ~31) * kR);
-  const uint64_t wq0 = (uint64_t)a.r0 + w_i0 - ((a.first && w_i0 > 0) ? 1u : 0u);
-  const uint32_t slot_w = (uint32_t)(wq0 / a.ss);                // warp-uniform
+  const WindowGrid g{a.ss, a.r0, a.first};
+  const uint32_t slot_a = g.slot(i0);
+  const uint32_t bnd = (uint32_t)g.end(slot_a);                  // first call-relative index of slot_a + 1
+  const uint32_t slot_w = g.slot((uint32_t)tile_base + (uint32_t)((tid & ~31) * kR));   // warp-uniform
+  // which of this thread's 8 outputs go to the upper of the warp's two windows (bit r), and which exist
+  uint32_t upper_mask = 0, valid_mask = 0;
+#pragma unroll
+  for (int r = 0; r < kR; ++r) {
+    const uint32_t i = i0 + r;
+    const bool up = (i >= bnd) ? (slot_a + 1 != slot_w) : (slot_a != slot_w);
+    upper_mask |= (up ? 1u : 0u) << r;
+    valid_mask |= ((i < tile_hi) ? 1u : 0u) << r;
+  }
 
   for (int ch = 0; ch < nch; ++ch) {
     const int c = c0 + ch;
-    const int4 *tpc = tp + ch * Lp;
     uint32_t A1[kR], A2[kR], A3[kR];
-    int wr[kR], wi[kR], ws[kR];
-#pragma unroll
-    for (int k = 0; k < kR; ++k) {
-      A1[k] = A2[k] = A3[k] = 0u;
-      unpack16(xs[pad32(ob + k)], wr[k], wi[k]);
-      ws[k] = wr[k] + wi[k];
-    }
-    for (int t0 = 0; t0 < Lp; t0 += kR) {
-#pragma unroll
-      for (int u = 0; u < kR; ++u) {
-        const int t = t0 + u;
-        if (t < Lp) {
-          const int4 cf = tpc[t];
-#pragma unroll
-          for (int r = 0; r < kR; ++r) {
-            const int s = (r + u) & (kR - 1);
-            A1[r] += (uint32_t)cf.x * (uint32_t)ws[s];
-            A2[r] += (uint32_t)cf.y * (uint32_t)wr[s];
-            A3[r] += (uint32_t)cf.z * (uint32_t)wi[s];
-          }
-          unpack16(xs[pad32(ob + t + kR)], wr[u], wi[u]);
-          ws[u] = wr[u] + wi[u];
-        }
-      }
-    }
+    fir_smem(xs, ob, tp + ch * Lp, Lp, A1, A2, A3);
     const uint32_t inc = a.inc[c] & 0x7fffu;
     const bool nco = a.inc[c] != 0, neg = (a.neg[c] != 0);
     const uint32_t phase0 = (a.consumed15 * inc) & 0x7fffu;      // (consumed * inc) mod 32768
     uint32_t lo_r = 0, lo_i = 0, hi_r = 0, hi_i = 0;             // sums for slot_w and slot_w + 1
 #pragma unroll
     for (int r = 0; r < kR; ++r) {
-      int yr = ((int)(A1[r] - A3[r])) >> 14;
-      int yi = ((int)(A1[r] + A2[r])) >> 14;
-      if (IS_S8) { yr = (int)(short)yr; yi = (int)(short)yi; }
+      int yr, yi;
+      fir_result<IS_S8, kFirComplex>(A1[r], A2[r], A3[r], 0u, 14, false, yr, yi);
       if (nco) {
         const uint32_t ph = (phase0 + (i0 + r) * inc) & 0x7fffu;
         uint32_t idx = ph >> 8;
         if (neg) idx = 127u - idx;
-        const int2 l = lut[idx];
-        const uint32_t pr = (uint32_t)l.x * (uint32_t)yr - (uint32_t)l.y * (uint32_t)yi;
-        const uint32_t pi = (uint32_t)l.x * (uint32_t)yi + (uint32_t)l.y * (uint32_t)yr;
-        if (IS_S8) { yr = (int)(short)(((int)(short)pr) >> 8); yi = (int)(short)(((int)(short)pi) >> 8); }
-        else { yr = ((int)pr) >> 16; yi = ((int)pi) >> 16; }
+        nco_mix<IS_S8>(lut[idx], yr, yi);
       }
-      const uint32_t i = i0 + r;
-      if (i < tile_hi) {
-        const bool upper = ((int64_t)i >= bnd) ? (slot_a + 1 != slot_w) : (slot_a != slot_w);
-        if (upper) { hi_r += (uint32_t)yr; hi_i += (uint32_t)yi; } else { lo_r += (uint32_t)yr; lo_i += (uint32_t)yi; }
+      if ((valid_mask >> r) & 1u) {
+        if ((upper_mask >> r) & 1u) { hi_r += (uint32_t)yr; hi_i += (uint32_t)yi; } else { lo_r += (uint32_t)yr; lo_i += (uint32_t)yi; }
       }
     }
     lo_r = __reduce_add_sync(kFull, lo_r); lo_i = __reduce_add_sync(kFull, lo_i);
@@ -166,21 +110,7 @@ __global__ void __launch_bounds__(kT) bank_accum_fixed_kernel(const BankAccumArg
   int4 *tp = (int4 *)(xs + ((n_xs + 3) & ~3));                   // group x LP
   int2 *lut = (int2 *)(tp + (size_t)a.group * LP);               // 128
 
-  {
-    int2 *nxt = (int2 *)a.acc_next;
-    const size_t total = (size_t)a.zero_next * a.channels;
-    const size_t stride = (size_t)gridDim.x * gridDim.y * blockDim.x;
-    for (size_t k = ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * blockDim.x + tid; k < total; k += stride)
-      nxt[(k / a.zero_next) * a.acc_stride + (k % a.zero_next)] = make_int2(0, 0);
-    if (blockIdx.x == 0 && blockIdx.y == 0) {
-      const int64_t n = a.n, Hh = a.hist_len;
-      for (int64_t k = tid; k < Hh; k += blockDim.x) {
-        const int64_t i = n - Hh + k;
-        if (IS_S8) ((char2 *)a.hist_out)[k] = (i >= 0) ? ((const char2 *)a.x)[i] : ((const char2 *)a.hist_in)[Hh + i];
-        else ((uint32_t *)a.hist_out)[k] = (i >= 0) ? ((const uint32_t *)a.x)[i] : ((const uint32_t *)a.hist_in)[Hh + i];
-      }
-    }
-  }
+  if (IS_S8) bank_prologue<char2>(a, tid); else bank_prologue<uint32_t>(a, tid);
 
   const int64_t tile_base = (int64_t)blockIdx.x * kTile;
   for (int k = tid; k < nch * LP; k += kT) {
@@ -189,20 +119,7 @@ __global__ void __launch_bounds__(kT) bank_accum_fixed_kernel(const BankAccumArg
   }
   if (tid < 128) lut[tid] = ((const int2 *)a.lut)[tid];
   const int Hh = (int)a.hist_len;
-  for (int k = tid; k < n_xs; k += kT) {
-    const int64_t i = tile_base - H + k;
-    uint32_t v = 0;
-    if (IS_S8) {
-      char2 s = make_char2(0, 0);
-      if (i < 0) { if (Hh + i >= 0) s = ((const char2 *)a.hist_in)[Hh + i]; }
-      else if (i < (int64_t)a.n) s = ((const char2 *)a.x)[i];
-      v = ((uint32_t)(uint16_t)(int16_t)s.x) | (((uint32_t)(uint16_t)(int16_t)s.y) << 16);
-    } else {
-      if (i < 0) { if (Hh + i >= 0) v = ((const uint32_t *)a.hist_in)[Hh + i]; }
-      else if (i < (int64_t)a.n) v = ((const uint32_t *)a.x)[i];
-    }
-    xs[k] = v;
-  }
+  for (int k = tid; k < n_xs; k += kT) xs[k] = load_sample<IS_S8>(a.x, a.hist_in, tile_base - H + k, Hh, a.n, 0u);
   __syncthreads();
 
   uint32_t w[4 * NV];
@@ -215,11 +132,10 @@ __global__ void __launch_bounds__(kT) bank_accum_fixed_kernel(const BankAccumArg
   const int ob = tid * kR;
   const uint32_t i0 = (uint32_t)tile_base + (uint32_t)ob;
   const uint32_t tile_hi = (uint32_t)min((int64_t)a.n, tile_base + kTile);
-  const uint32_t q0 = a.r0 + i0 - ((a.first && i0 > 0) ? 1u : 0u);
-  const uint32_t slot_a = q0 / a.ss;
-  const uint32_t bnd = (slot_a + 1) * a.ss - a.r0 + a.first;      // first index of slot_a + 1
-  const uint32_t w_i0 = (uint32_t)tile_base + (uint32_t)((tid & ~31) * kR);
-  const uint32_t slot_w = (a.r0 + w_i0 - ((a.first && w_i0 > 0) ? 1u : 0u)) / a.ss;
+  const WindowGrid g{a.ss, a.r0, a.first};
+  const uint32_t slot_a = g.slot(i0);
+  const uint32_t bnd = (uint32_t)g.end(slot_a);                  // first index of slot_a + 1
+  const uint32_t slot_w = g.slot((uint32_t)tile_base + (uint32_t)((tid & ~31) * kR));
   // which of this thread's 8 outputs go to the upper of the warp's two windows (bit r), and which exist
   uint32_t upper_mask = 0, valid_mask = 0;
 #pragma unroll
@@ -232,30 +148,8 @@ __global__ void __launch_bounds__(kT) bank_accum_fixed_kernel(const BankAccumArg
 
   for (int ch = 0; ch < nch; ++ch) {
     const int c = c0 + ch;
-    const int4 *tpc = tp + ch * LP;
     uint32_t A1[kR], A2[kR], A3[kR];
-    int wr[kR], wi[kR], ws[kR];
-#pragma unroll
-    for (int k = 0; k < kR; ++k) {
-      A1[k] = A2[k] = A3[k] = 0u;
-      unpack16(w[k], wr[k], wi[k]);
-      ws[k] = wr[k] + wi[k];
-    }
-#pragma unroll
-    for (int t = 0; t < LP; ++t) {
-      const int4 cf = tpc[t];
-#pragma unroll
-      for (int r = 0; r < kR; ++r) {
-        const int s = (r + t) & (kR - 1);
-        A1[r] += (uint32_t)cf.x * (uint32_t)ws[s];
-        A2[r] += (uint32_t)cf.y * (uint32_t)wr[s];
-        A3[r] += (uint32_t)cf.z * (uint32_t)wi[s];
-      }
-      if (t + 1 < LP) {
-        unpack16(w[t + kR], wr[t & (kR - 1)], wi[t & (kR - 1)]);
-        ws[t & (kR - 1)] = wr[t & (kR - 1)] + wi[t & (kR - 1)];
-      }
-    }
+    fir_fixed<LP, kFirComplex>(w, tp + ch * LP, 0u, A1, A2, A3);
     const uint32_t inc = a.inc[c] & 0x7fffu;
     const bool nco = a.inc[c] != 0;
     const uint32_t negx = a.neg[c] ? 127u : 0u;                  // idx = 127 - idx  <=>  idx ^ 127 for idx in 0..127
@@ -263,16 +157,12 @@ __global__ void __launch_bounds__(kT) bank_accum_fixed_kernel(const BankAccumArg
     uint32_t lo_r = 0, lo_i = 0, hi_r = 0, hi_i = 0;
 #pragma unroll
     for (int r = 0; r < kR; ++r) {
-      int yr = ((int)(A1[r] - A3[r])) >> 14;
-      int yi = ((int)(A1[r] + A2[r])) >> 14;
-      if (IS_S8) { yr = (int)(short)yr; yi = (int)(short)yi; }
+      int yr, yi;
+      fir_result<IS_S8, kFirComplex>(A1[r], A2[r], A3[r], 0u, 14, false, yr, yi);
       if (nco) {
         const int2 l = lut[(ph >> 8) ^ negx];
         ph = (ph + inc) & 0x7fffu;
-        const uint32_t pr = (uint32_t)l.x * (uint32_t)yr - (uint32_t)l.y * (uint32_t)yi;
-        const uint32_t pi = (uint32_t)l.x * (uint32_t)yi + (uint32_t)l.y * (uint32_t)yr;
-        if (IS_S8) { yr = (int)(short)(((int)(short)pr) >> 8); yi = (int)(short)(((int)(short)pi) >> 8); }
-        else { yr = ((int)pr) >> 16; yi = ((int)pi) >> 16; }
+        nco_mix<IS_S8>(l, yr, yi);
       }
       if ((valid_mask >> r) & 1u) {
         if ((upper_mask >> r) & 1u) { hi_r += (uint32_t)yr; hi_i += (uint32_t)yi; } else { lo_r += (uint32_t)yr; lo_i += (uint32_t)yi; }

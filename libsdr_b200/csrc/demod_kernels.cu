@@ -73,13 +73,6 @@ __global__ void __launch_bounds__(256) envelope_kernel(const typename In<SCALAR>
   }
 }
 
-// AutoCast< complex<int16_t> > (src/autocast.hh:187-204), one byte per thread-iteration
-__global__ void __launch_bounds__(256) autocast_cs16_kernel(const signed char *in, size_t n, short *out, int bias) {
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
-    out[i] = (short)(((int)in[i] - bias) << 8);
-}
-
 // FMDeemph<int16_t> (src/demod.hh:345-352): a 1-pole integer IIR with rounding -- serial and not
 // associative within a stream, so one thread walks one stream; banks give the parallelism.
 __global__ void __launch_bounds__(128) fmdeemph_kernel(const short *in, short *out, size_t n, size_t streams, size_t stride,
@@ -134,14 +127,6 @@ static int launch_envelope(int scalar, const void *in, size_t n, void *out, cuda
     default: return set_error(SDRG_ERR_ARG, "demod: unsupported scalar %d", scalar);
   }
   SDRG_CHECK_LAUNCH(USB ? "usbdemod_kernel" : "amdemod_kernel");
-  return SDRG_OK;
-}
-
-int launch_autocast_cs16(int fmt, const void *in, size_t n_bytes, void *out, cudaStream_t st) {
-  if (n_bytes == 0) return SDRG_OK;
-  if (fmt != 2 && fmt != 3) return set_error(SDRG_ERR_ARG, "AutoCast: unsupported input format %d", fmt);
-  autocast_cs16_kernel<<<grid_for(n_bytes), 256, 0, st>>>((const signed char *)in, n_bytes, (short *)out, fmt == 2 ? 127 : 0);
-  SDRG_CHECK_LAUNCH("autocast_cs16_kernel");
   return SDRG_OK;
 }
 

@@ -27,11 +27,6 @@ __device__ __forceinline__ void cfma(float2 &acc, float2 w, float2 x) {
   acc = __ffma2_rn(x, make_float2(w.x, w.x), acc);
   acc = __ffma2_rn(make_float2(-x.y, x.x), make_float2(w.y, w.y), acc);
 }
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(kFull, v, d);
-  return v;
-}
 __device__ __forceinline__ void flush(float *acc, uint32_t slot, float2 v, int lane) {
   const float sr = warp_sum(v.x), si = warp_sum(v.y);
   if (lane == 0 && (sr != 0.f || si != 0.f)) { atomicAdd(acc + 2 * (size_t)slot, sr); atomicAdd(acc + 2 * (size_t)slot + 1, si); }

@@ -45,8 +45,6 @@ struct PerwinGeom {
 __device__ __forceinline__ void cp_async8(float2 *dst_smem, const float2 *src) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((uint32_t)__cvta_generic_to_shared(dst_smem)), "l"(src) : "memory");
 }
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // 1-D bulk async copies (TMA, SASS UBLKCP) completing on an mbarrier: the staging of the half-warp kernels costs no
 // LSU issue slots and no registers (an 8-byte LDGSTS occupies the LSU pipe for ~8 cycles per warp instruction)

@@ -25,28 +25,11 @@ namespace sdrg {
 namespace {
 
 constexpr int kT = kIqbbThreads;
-constexpr int kR = kIqbbPerThread;
 constexpr int kTile = kIqbbTile;
 constexpr int kZRow = kT + 2;              // row pitch of the transposed z staging (bank spread)
 constexpr unsigned kFull = 0xffffffffu;
 
-__device__ __forceinline__ int pad32(int i) { return i + (i >> 5); }   // 4-byte elements, 8 per thread
 __device__ __forceinline__ int pad64(int i) { return i + (i >> 3); }   // 8-byte elements, 8 per thread
-
-// window bookkeeping (call-relative sample index i): q(i) = r0 + i - (first && i>0); slot = q/ss.
-// n <= 2^30 and r0 < ss <= 2^30, so q and every window bound fit in 32 bits (the 64-bit division
-// this used to be cost more than the FIR itself).
-struct WindowGrid {
-  uint32_t ss, r0, first;
-  __device__ __forceinline__ uint32_t q(uint32_t i) const { return r0 + i - ((first && i > 0) ? 1u : 0u); }
-  __device__ __forceinline__ uint32_t slot(uint32_t i) const { return q(i) / ss; }
-  __device__ __forceinline__ int64_t begin(uint32_t s) const {
-    return s == 0 ? 0 : (int64_t)(uint32_t)(s * ss - r0 + first);
-  }
-  __device__ __forceinline__ int64_t end(uint32_t s) const {
-    return (int64_t)(uint32_t)((s + 1) * ss - r0 + first);
-  }
-};
 
 // Per-window partial sums of one tile from the transposed z staging, added into the call's
 // accumulators.  Short windows (ss <= 64: >= 32 windows per tile) take one THREAD per window --
@@ -87,9 +70,7 @@ __device__ __forceinline__ void window_sums_int(const IqbbAccumArgs &a, const in
   }
 }
 
-// ---- integer kernel ------------------------------------------------------------------------------
-// taps: int4 {kr, ki-kr, kr+ki, 0} per tap (Gauss: t1=kr(xr+xi), t2=(ki-kr)xr, t3=(kr+ki)xi;
-// re=t1-t3, im=t1+t2 -- ring identities, hence exact mod 2^32).
+// ---- integer kernel (arithmetic: iqbb_int_common.cuh) ---------------------------------------------
 template <bool IS_S8>
 __global__ void __launch_bounds__(kT) iqbb_accum_int_kernel(const IqbbAccumArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -107,83 +88,25 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_kernel(const IqbbAccumArgs 
   // stage taps / LUT / samples
   for (int k = tid; k < Lp; k += kT) tp[k] = ((const int4 *)a.taps)[k];
   if (tid < 128) lut[tid] = ((const int2 *)a.lut)[tid];
-  for (int k = tid; k < n_xs; k += kT) {
-    const int64_t i = tile_base - H + k;
-    uint32_t v = 0;
-    if (IS_S8 && a.in_fmt == 5) {                                // BaseBand<int8_t>: real samples, (x, 0)
-      signed char s = 0;
-      if (i < 0) s = ((const signed char *)a.hist_in)[H + i];
-      else if (i < (int64_t)a.n) s = ((const signed char *)a.x)[i];
-      v = (uint32_t)(uint16_t)(int16_t)s;
-    } else if (IS_S8) {
-      char2 s = make_char2(0, 0);
-      if (i < 0) s = ((const char2 *)a.hist_in)[H + i];
-      else if (i < (int64_t)a.n) s = ((const char2 *)a.x)[i];
-      v = ((uint32_t)(uint16_t)(int16_t)s.x) | (((uint32_t)(uint16_t)(int16_t)s.y) << 16);
-    } else {
-      if (i < 0) v = load_cs16(a.hist_in, H + i, a.in_fmt);
-      else if (i < (int64_t)a.n) v = load_cs16(a.x, i, a.in_fmt);
-    }
-    xs[pad32(k)] = v;
-  }
+  for (int k = tid; k < n_xs; k += kT) xs[pad32(k)] = load_sample<IS_S8>(a.x, a.hist_in, tile_base - H + k, H, a.n, a.in_fmt);
   __syncthreads();
 
   // FIR: outputs ob..ob+7 of the tile; window sample c lives at xs[ob + c]
   const int ob = tid * kR;
   uint32_t A1[kR], A2[kR], A3[kR];
-  int wr[kR], wi[kR], ws[kR];
-#pragma unroll
-  for (int c = 0; c < kR; ++c) {
-    A1[c] = A2[c] = A3[c] = 0u;
-    unpack16(xs[pad32(ob + c)], wr[c], wi[c]);
-    ws[c] = wr[c] + wi[c];
-  }
-  for (int t0 = 0; t0 < Lp; t0 += kR) {
-#pragma unroll
-    for (int u = 0; u < kR; ++u) {
-      const int t = t0 + u;
-      if (t < Lp) {
-        const int4 c = tp[t];
-#pragma unroll
-        for (int r = 0; r < kR; ++r) {
-          const int s = (r + u) & (kR - 1);
-          A1[r] += (uint32_t)c.x * (uint32_t)ws[s];
-          A2[r] += (uint32_t)c.y * (uint32_t)wr[s];
-          A3[r] += (uint32_t)c.z * (uint32_t)wi[s];
-        }
-        unpack16(xs[pad32(ob + t + kR)], wr[u], wi[u]);   // slot u is dead now: next window sample
-        ws[u] = wr[u] + wi[u];
-      }
-    }
-  }
+  fir_smem(xs, ob, tp, Lp, A1, A2, A3);
 
-  // >>14, NCO, stage z (transposed: row r, column tid)
+  // >> fir_shift, NCO, stage z (transposed: row r, column tid)
   const uint32_t i0 = (uint32_t)tile_base + (uint32_t)ob;
 #pragma unroll
   for (int r = 0; r < kR; ++r) {
     int yr, yi;
-    if (IS_S8 && a.in_fmt == 5) {     // BaseBand<int8_t>: `res` is complex<int16_t>, the sum wraps at 16 bits, then >> 8
-      yr = ((int)(short)(A1[r] - A3[r])) >> a.fir_shift;
-      yi = ((int)(short)(A1[r] + A2[r])) >> a.fir_shift;
-    } else {
-      yr = ((int)(A1[r] - A3[r])) >> a.fir_shift;
-      yi = ((int)(A1[r] + A2[r])) >> a.fir_shift;
-    }
-    if (IS_S8) { yr = (int)(short)yr; yi = (int)(short)yi; }   // narrowed to complex<int16_t> on the call
+    fir_result<IS_S8, kFirComplex>(A1[r], A2[r], A3[r], 0u, a.fir_shift, IS_S8 && a.in_fmt == 5, yr, yi);
     if (a.nco) {
       const uint32_t ph = (a.phase0 + (i0 + r) * a.inc) & 0x7fffu;
       uint32_t idx = ph >> 8;
       if (a.neg) idx = 127u - idx;
-      const int2 l = lut[idx];
-      const uint32_t pr = (uint32_t)l.x * (uint32_t)yr - (uint32_t)l.y * (uint32_t)yi;
-      const uint32_t pi = (uint32_t)l.x * (uint32_t)yi + (uint32_t)l.y * (uint32_t)yr;
-      if (IS_S8) {   // product narrowed to int16, shifted by 8, narrowed again (freqshift.hh:67)
-        yr = (int)(short)(((int)(short)pr) >> 8);
-        yi = (int)(short)(((int)(short)pi) >> 8);
-      } else {
-        yr = ((int)pr) >> 16;
-        yi = ((int)pi) >> 16;
-      }
+      nco_mix<IS_S8>(lut[idx], yr, yi);
     }
     zs[r * kZRow + tid] = make_int2(yr, yi);
   }
@@ -193,9 +116,9 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_kernel(const IqbbAccumArgs 
 }
 
 // ---- integer kernel, compile-time tap count -------------------------------------------------------
-// Same arithmetic as above with the tap count LP fixed at compile time (taps zero-padded at the
-// FRONT to the next even count, which is exact): the tile is staged unpadded, every thread pulls
-// its LP+7 packed samples with 128-bit shared loads into registers ONCE, the taps sit in the
+// The tap count LP is fixed at compile time (taps zero-padded at the FRONT to the next even count,
+// which is exact): the tile is staged unpadded, every thread pulls its LP+7 packed samples
+// with 128-bit shared loads into registers ONCE, the taps sit in the
 // kernel's parameter (constant) bank so the FIR inner loop is nothing but IMADs with a constant
 // operand plus one unpack per sample -- no loads, no guards, no address arithmetic.
 // Persistent CTAs (one per resident slot) walk the tiles grid-stride; the next tile is fetched into
@@ -205,7 +128,7 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_kernel(const IqbbAccumArgs 
 // the imaginary input is 0, so the Gauss form collapses to two multiplies per tap: re = sum kr x, im = re + sum (ki-kr) x).
 template <int LP, int VAR>
 __global__ void __launch_bounds__(kT) iqbb_accum_int_fixed_kernel(const IqbbAccumArgs a, const __grid_constant__ IqbbTaps taps) {
-  constexpr bool IS_S8 = VAR == 1, REAL = VAR == 2;
+  constexpr bool IS_S8 = VAR == 1;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   constexpr int H = LP - 1;
   constexpr int NV = (LP + 7 + 3) / 4;                 // 128-bit loads per thread
@@ -219,6 +142,7 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_fixed_kernel(const IqbbAccu
   if (IS_S8) prologue<char2, int2>(a); else prologue<short2, int2>(a);
   if (tid < 128) lut[tid] = ((const int2 *)a.lut)[tid];
   const int Hh = (int)a.hist_len;                                // history kept by the handle (= stripped taps - 1 <= H)
+  const uint32_t fmt = IS_S8 ? 0u : a.in_fmt;                    // int8 here is complex (BaseBand<int8_t> takes the generic kernel)
   const uint32_t n_tiles = (a.n + kTile - 1) / kTile;
 
   // stage tile t into xs: asynchronously when it is an interior int16 tile, synchronously otherwise
@@ -232,20 +156,7 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_fixed_kernel(const IqbbAccu
       const int64_t i0 = tile_base - H;
       for (int k = tid; k < n_xs; k += kT) xs[k] = load_cs16(a.x, i0 + k, a.in_fmt);
     } else {
-      for (int k = tid; k < n_xs; k += kT) {
-        const int64_t i = tile_base - H + k;
-        uint32_t v = 0;
-        if (IS_S8) {
-          char2 s = make_char2(0, 0);
-          if (i < 0) { if (Hh + i >= 0) s = ((const char2 *)a.hist_in)[Hh + i]; }
-          else if (i < (int64_t)a.n) s = ((const char2 *)a.x)[i];
-          v = ((uint32_t)(uint16_t)(int16_t)s.x) | (((uint32_t)(uint16_t)(int16_t)s.y) << 16);
-        } else {
-          if (i < 0) { if (Hh + i >= 0) v = load_cs16(a.hist_in, Hh + i, a.in_fmt); }
-          else if (i < (int64_t)a.n) v = load_cs16(a.x, i, a.in_fmt);
-        }
-        xs[k] = v;
-      }
+      for (int k = tid; k < n_xs; k += kT) xs[k] = load_sample<IS_S8>(a.x, a.hist_in, tile_base - H + k, Hh, a.n, fmt);
     }
     cp_async_commit();
   };
@@ -265,34 +176,9 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_fixed_kernel(const IqbbAccu
       const uint4 q = ((const uint4 *)xs)[tid * 2 + v];
       w[4 * v] = q.x; w[4 * v + 1] = q.y; w[4 * v + 2] = q.z; w[4 * v + 3] = q.w;
     }
+    constexpr int FORM = VAR == 2 ? kFirRealIn : kFirComplex;
     uint32_t A1[kR], A2[kR], A3[kR];
-    int wr[kR], wi[kR], ws[kR];
-#pragma unroll
-    for (int c = 0; c < kR; ++c) {
-      A1[c] = A2[c] = A3[c] = 0u;
-      unpack16(w[c], wr[c], wi[c]);
-      ws[c] = wr[c] + wi[c];
-    }
-#pragma unroll
-    for (int tt = 0; tt < LP; ++tt) {
-      const int4 c = taps.t[tt];
-#pragma unroll
-      for (int r = 0; r < kR; ++r) {
-        const int s = (r + tt) & (kR - 1);
-        if (REAL) {
-          A1[r] += (uint32_t)c.x * (uint32_t)wr[s];
-          A2[r] += (uint32_t)c.y * (uint32_t)wr[s];
-        } else {
-          A1[r] += (uint32_t)c.x * (uint32_t)ws[s];
-          A2[r] += (uint32_t)c.y * (uint32_t)wr[s];
-          A3[r] += (uint32_t)c.z * (uint32_t)wi[s];
-        }
-      }
-      if (tt + 1 < LP) {
-        unpack16(w[tt + kR], wr[tt & (kR - 1)], wi[tt & (kR - 1)]);
-        ws[tt & (kR - 1)] = wr[tt & (kR - 1)] + wi[tt & (kR - 1)];
-      }
-    }
+    fir_fixed<LP, FORM>(w, taps.t, 0u, A1, A2, A3);
 
     const int ob = tid * kR;
     const uint32_t i0 = (uint32_t)tile_base + (uint32_t)ob;
@@ -300,16 +186,12 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_fixed_kernel(const IqbbAccu
     uint32_t ph = (a.phase0 + i0 * a.inc) & 0x7fffu;
 #pragma unroll
     for (int r = 0; r < kR; ++r) {
-      int yr = ((int)(A1[r] - A3[r])) >> a.fir_shift;
-      int yi = ((int)(A1[r] + A2[r])) >> a.fir_shift;
-      if (IS_S8) { yr = (int)(short)yr; yi = (int)(short)yi; }
+      int yr, yi;
+      fir_result<IS_S8, FORM>(A1[r], A2[r], A3[r], 0u, a.fir_shift, false, yr, yi);
       if (a.nco) {
         const int2 l = lut[(ph >> 8) ^ negx];
         ph = (ph + a.inc) & 0x7fffu;
-        const uint32_t pr = (uint32_t)l.x * (uint32_t)yr - (uint32_t)l.y * (uint32_t)yi;
-        const uint32_t pi = (uint32_t)l.x * (uint32_t)yi + (uint32_t)l.y * (uint32_t)yr;
-        if (IS_S8) { yr = (int)(short)(((int)(short)pr) >> 8); yi = (int)(short)(((int)(short)pi) >> 8); }
-        else { yr = ((int)pr) >> 16; yi = ((int)pi) >> 16; }
+        nco_mix<IS_S8>(l, yr, yi);
       }
       zs[r * kZRow + tid] = make_int2(yr, yi);
     }
@@ -333,12 +215,6 @@ int dispatch_fixed(int lp, const IqbbAccumArgs &a, const IqbbTaps &taps, unsigne
 }
 
 // ---- float kernel (direct form; the folded fast path lives in iqbb_fold_kernels.cu) ---------------
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(kFull, v, d);
-  return v;
-}
-
 __global__ void __launch_bounds__(kT) iqbb_accum_f32_kernel(const IqbbAccumArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;

@@ -8,6 +8,17 @@ constexpr int kIqbbThreads = 256;      // threads per CTA of the accumulate kern
 constexpr int kIqbbPerThread = 8;      // consecutive FIR outputs per thread (register blocking)
 constexpr int kIqbbTile = kIqbbThreads * kIqbbPerThread;   // input samples per CTA
 
+// ---- device helpers of the integer and float accumulate kernels ----------------------------------
+namespace {
+__device__ __forceinline__ float warp_sum(float v) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) v += __shfl_xor_sync(0xffffffffu, v, d);
+  return v;
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+}  // namespace
+
 // One process() call of the direct (unfolded) kernels.  All indices are relative to the first
 // sample of the call; the host carries the global position (closed form, SURVEY.md 8 a1/a2).
 struct IqbbAccumArgs {
@@ -117,8 +128,6 @@ int launch_fmdemod(int scalar, const void *in, size_t n, void *out, const void *
                    int in_place, cudaStream_t st);
 int launch_amdemod(int scalar, const void *in, size_t n, void *out, cudaStream_t st);
 int launch_usbdemod(int scalar, const void *in, size_t n, void *out, cudaStream_t st);
-// AutoCast<complex<int16_t>> from complex uint8 (fmt 2) / int8 (fmt 3): n_bytes in, n_bytes int16 out
-int launch_autocast_cs16(int fmt, const void *in, size_t n_bytes, void *out, cudaStream_t st);
 // the whole AutoCast table: kind 1..14 (demod_kernels.cu), n_scalars input scalars
 int launch_autocast(int kind, const void *in, size_t n_scalars, void *out, cudaStream_t st);
 // FMDeemph<int16_t>: `streams` independent sequences of n samples (stride elements apart), one thread each

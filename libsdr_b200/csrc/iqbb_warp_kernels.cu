@@ -1,16 +1,17 @@
 // iqbb_warp_kernels.cu -- IQBaseBand<int16_t>/<int8_t>, fixed tap count, one WARP per 256-sample tile and no CTA
 // barrier anywhere in the loop.
 //
-// Same arithmetic as iqbb_accum_int_fixed_kernel (iqbb_kernels.cu; reference src/baseband.hh:198-236, bit-exact:
-// every sum is taken in Z/2^32).  What changed is the choreography.  The CTA-wide kernel staged 2048 samples for 256
-// threads, exchanged the mixed samples through a transposed shared array and summed each window with one thread or
-// one warp -- two __syncthreads per tile, 41 of 256 threads busy in the window phase at sub_sample 50, and the barrier
-// was the top stall (profiles/r01_final_int16_kernel_summary.md: 59 % of the IMAD pipe against the bank kernel's 86 %).
+// The arithmetic is iqbb_int_common.cuh's (load_sample, fir_fixed, fir_result, nco_mix, narrow16), as in
+// iqbb_accum_int_fixed_kernel; only the symmetric-tap FIR (VAR 4) is this kernel's own, and int8's narrowing to int16
+// is applied just before the NCO mix rather than inside fir_result.  What changed is the choreography.  The CTA-wide
+// kernel staged 2048 samples for 256 threads, exchanged the mixed samples through a transposed shared array and summed
+// each window with one thread or one warp -- two __syncthreads per tile, 41 of 256 threads busy in the window phase at
+// sub_sample 50, and the barrier was the top stall (profiles/r01_final_int16_kernel_summary.md: 59 % of the IMAD pipe against the bank kernel's 86 %).
 // Here a warp owns its tile end to end:
 //   * it stages its own 256 + LP + 7 samples with cp.async into a private, double-buffered shared region (the next
 //     tile is in flight while the current one is filtered), 16-byte chunks XOR-swizzled so that the 128-bit reads
 //     of lanes j and j + 4 no longer collide;
-//   * FIR (taps in the constant bank) and NCO run out of registers exactly as before;
+//   * FIR (taps in the constant bank) and NCO run out of registers as in the CTA-wide kernel;
 //   * the window sums never leave the warp: a lane's 8 consecutive outputs touch at most two windows
 //     (sub_sample >= 16), so it forms two partial sums and adds them to a per-warp shared accumulator line
 //     (native shared-memory integer atomics; their serialisation costs LSU cycles, not IMAD-pipe slots), or, when
@@ -27,7 +28,6 @@ namespace sdrg {
 namespace {
 
 constexpr int kT = kIqbbThreads;           // 8 warps per CTA
-constexpr int kR = kIqbbPerThread;         // 8 outputs per lane
 constexpr int kWT = 32 * kR;               // outputs per warp tile
 constexpr unsigned kFull = 0xffffffffu;
 
@@ -41,7 +41,8 @@ __device__ __forceinline__ uint32_t div_ss(uint32_t q, uint32_t m, uint32_t s) {
 // so that the plain complex int16 path does not carry the staging registers.
 template <int LP, int VAR, bool CONV>
 __global__ void __launch_bounds__(kT) iqbb_accum_int_warp_kernel(const IqbbAccumArgs a, const __grid_constant__ IqbbTaps taps) {
-  constexpr bool IS_S8 = VAR == 1, REAL_IN = VAR == 2, REAL_TAPS = VAR == 3, SYM = VAR == 4;
+  constexpr bool IS_S8 = VAR == 1, SYM = VAR == 4;
+  constexpr int FORM = VAR == 2 ? kFirRealIn : VAR == 3 ? kFirRealTaps : kFirComplex;
   constexpr int H = LP - 1;
   constexpr int NV = (LP + 7 + 3) / 4;                 // 128-bit loads per lane
   constexpr int n_xs = kWT - kR + 4 * NV;              // words a warp tile needs: lane 31 reads [248, 248 + 4 NV)
@@ -60,6 +61,7 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_warp_kernel(const IqbbAccum
   __syncthreads();                                                     // the only CTA barrier: LUT and accumulators are in place
 
   const int Hh = (int)a.hist_len;                                      // history the handle keeps (stripped taps - 1 <= H)
+  const uint32_t fmt = IS_S8 ? 0u : a.in_fmt;                          // int8 here is complex
   const uint32_t Z = a.zero;                                           // == 0; see IqbbAccumArgs::zero
   const uint32_t n_tiles = (a.n + kWT - 1) / kWT;
   const uint32_t n_warps = gridDim.x * (kT / 32);
@@ -82,20 +84,7 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_warp_kernel(const IqbbAccum
       for (int j = 0; j < NL; ++j) { const int k = lane + 32 * j; raw[j] = k < n_xs ? load_cs16(a.x, base + k, a.in_fmt) : 0u; }
       raw_pending = true;
     } else {
-      for (int k = lane; k < n_xs; k += 32) {
-        const int64_t i = base + k;
-        uint32_t v = 0;
-        if (IS_S8) {
-          char2 s = make_char2(0, 0);
-          if (i < 0) { if (Hh + i >= 0) s = ((const char2 *)a.hist_in)[Hh + i]; }
-          else if (i < (int64_t)a.n) s = ((const char2 *)a.x)[i];
-          v = ((uint32_t)(uint16_t)(int16_t)s.x) | (((uint32_t)(uint16_t)(int16_t)s.y) << 16);
-        } else {
-          if (i < 0) { if (Hh + i >= 0) v = load_cs16(a.hist_in, Hh + i, a.in_fmt); }
-          else if (i < (int64_t)a.n) v = load_cs16(a.x, i, a.in_fmt);
-        }
-        xs[(swz(k >> 2) << 2) | (k & 3)] = v;
-      }
+      for (int k = lane; k < n_xs; k += 32) xs[(swz(k >> 2) << 2) | (k & 3)] = load_sample<IS_S8>(a.x, a.hist_in, base + k, Hh, a.n, fmt);
     }
     cp_async_commit();
   };
@@ -141,64 +130,32 @@ __global__ void __launch_bounds__(kT) iqbb_accum_int_warp_kernel(const IqbbAccum
         }
       }
 #pragma unroll
-      for (int r = 0; r < kR; ++r) { yr[r] = ((int)Ar[r]) >> a.fir_shift; yi[r] = ((int)Ai[r]) >> a.fir_shift; }
+      for (int r = 0; r < kR; ++r) fir_result<false, kFirRealTaps>(Ar[r], Ai[r], 0u, 0u, a.fir_shift, false, yr[r], yi[r]);
     } else {
       uint32_t A1[kR], A2[kR], A3[kR];
-      int wr[kR], wi[kR], ws[kR];
+      fir_fixed<LP, FORM>(w, taps.t, Z, A1, A2, A3);
 #pragma unroll
-      for (int c = 0; c < kR; ++c) {
-        A1[c] = A2[c] = A3[c] = 0u;
-        unpack16(w[c], wr[c], wi[c]);
-        ws[c] = (int)((uint32_t)wr[c] + (uint32_t)wi[c] + Z);
-      }
-#pragma unroll
-      for (int tt = 0; tt < LP; ++tt) {
-        const int4 c = taps.t[tt];
-#pragma unroll
-        for (int r = 0; r < kR; ++r) {
-          const int s = (r + tt) & (kR - 1);
-          if (REAL_IN) {                       // sample = (x, 0): re = sum kr x, im = re + sum (ki - kr) x
-            A1[r] += (uint32_t)c.x * (uint32_t)wr[s];
-            A2[r] += (uint32_t)c.y * (uint32_t)wr[s];
-          } else if (REAL_TAPS) {              // tap = (kr, 0): re = sum kr xr, im = sum kr xi
-            A1[r] += (uint32_t)c.x * (uint32_t)wr[s];
-            A2[r] += (uint32_t)c.x * (uint32_t)wi[s];
-          } else {
-            A1[r] += (uint32_t)c.x * (uint32_t)ws[s];
-            A2[r] += (uint32_t)c.y * (uint32_t)wr[s];
-            A3[r] += (uint32_t)c.z * (uint32_t)wi[s];
-          }
-        }
-        if (tt + 1 < LP) {
-          unpack16(w[tt + kR], wr[tt & (kR - 1)], wi[tt & (kR - 1)]);
-          if (!REAL_IN && !REAL_TAPS) ws[tt & (kR - 1)] = (int)((uint32_t)wr[tt & (kR - 1)] + (uint32_t)wi[tt & (kR - 1)] + Z);
-        }
-      }
-#pragma unroll
-      for (int r = 0; r < kR; ++r) {
-        if (REAL_TAPS) { yr[r] = ((int)A1[r]) >> a.fir_shift; yi[r] = ((int)A2[r]) >> a.fir_shift; }
-        else { yr[r] = ((int)(A1[r] - A3[r] + Z)) >> a.fir_shift; yi[r] = ((int)(A1[r] + A2[r] + Z)) >> a.fir_shift; }
-      }
+      for (int r = 0; r < kR; ++r) fir_result<false, FORM>(A1[r], A2[r], A3[r], Z, a.fir_shift, false, yr[r], yi[r]);
     }
 
     // ---- NCO (in place on yr/yi).  The running phase is not masked: only bits 8..14 select the LUT entry.
+    // int8: fir_result's narrowing to int16 is applied here, just before the mix, which keeps this kernel's register
+    // allocation (the result is the same).
     const uint32_t i_w = wt * kWT, i0 = i_w + (uint32_t)lane * kR;
     if (a.nco) {
       uint32_t ph = a.phase0 + i0 * a.inc;
 #pragma unroll
       for (int r = 0; r < kR; ++r) {
         int zr = yr[r], zi = yi[r];
-        if (IS_S8) { zr = (int)(short)zr; zi = (int)(short)zi; }
+        if (IS_S8) narrow16(zr, zi);
         const int2 l = lut[(ph >> 8) & 127u];                          // (the table is staged reversed for negative shifts)
         ph += a.inc + Z;
-        const uint32_t pr = (uint32_t)l.x * (uint32_t)zr - (uint32_t)l.y * (uint32_t)zi;
-        const uint32_t pi = (uint32_t)l.x * (uint32_t)zi + (uint32_t)l.y * (uint32_t)zr;
-        if (IS_S8) { yr[r] = (int)(short)(((int)(short)pr) >> 8); yi[r] = (int)(short)(((int)(short)pi) >> 8); }
-        else { yr[r] = ((int)pr) >> 16; yi[r] = ((int)pi) >> 16; }
+        nco_mix<IS_S8>(l, zr, zi);
+        yr[r] = zr; yi[r] = zi;
       }
     } else if (IS_S8) {
 #pragma unroll
-      for (int r = 0; r < kR; ++r) { yr[r] = (int)(short)yr[r]; yi[r] = (int)(short)yi[r]; }
+      for (int r = 0; r < kR; ++r) narrow16(yr[r], yi[r]);
     }
 
     // ---- the lane's two partial window sums: `tot` over its valid outputs, `hi` over those past the window boundary
